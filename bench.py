@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                  # headline: cfg3, our arm (libblr_cuda on B200)
     python bench.py --config cfg2|cfg3|cfg4|cfg5 ...               # the other BASELINE configs, same one-line contract
     python bench.py --impl reference [--config ...] ...            # the reference's CPU op sequence on the box's host cores
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's results as DIR/<name>.npy
 
 Configs (BASELINE.json `configs`):
   cfg3  diagonal-noise BLR posterior+logpdf, N = 2^24, D = 1024, ColVecs, N-sharded (the config `metric` is quoted on; default)
@@ -19,6 +20,12 @@ collective is ONE NCCL sum-allreduce of the packed statistics per step (none on 
 checks its result -- posterior+logpdf configs against the committed log marginal likelihood of the same synthetic data set
 (profiles/bench_expected.json, relative 1e-11: the value must not depend on the number of GPUs), cfg4 against torch on
 sampled blocks of test points -- and exits non-zero on a mismatch.
+
+--dump-outputs DIR (rank 0, our arm): after the timed steps, the arrays the timed path returned in its LAST step, float64,
+one DIR/<name>.npy each -- posterior+logpdf configs: posterior_mean, posterior_precision, logpdf; cfg4: mean, var, rand
+(device draws), rand_supplied_draws.  An array of more than 2^20 elements is stored as its values at a fixed seeded set of
+flat (row-major) positions, the same for every run of the same shape, so that two builds can be compared output for
+output; the inputs are generated from --seed alone.  cfg4 with several GPUs dumps rank 0's shard of the test points.
 """
 from __future__ import annotations
 
@@ -41,6 +48,7 @@ sys.path.insert(0, ROOT)
 NOMINAL_FP64_TFLOPS = 37.2  # 148 SM x 64 DFMA/clk x 2 x 1.965 GHz (BASELINE.md)
 EXPECTED_PATH = os.path.join(ROOT, "profiles", "bench_expected.json")
 TRAFFIC_PATH = os.path.join(ROOT, "profiles", "gram_traffic.json")
+DUMP_MAX_ELEMS = 1 << 20  # 8 MiB of float64 per dumped array; at most four arrays per config keep a dump under 64 MB
 
 CONFIGS = {
     "cfg3": dict(kind="infer", n=1 << 24, dim=1024, unit="obs/s", metric="obs/s for posterior+logpdf (fp64, N=16M, D=1024)"),
@@ -506,6 +514,27 @@ def fill_tiled(torch, dst, gen, block_rows=1 << 16):
         dst[a:b].copy_(blk[: b - a])
 
 
+def dump_sample(x):
+    """A result array (numpy, or a torch tensor on any device) as float64 numpy for --dump-outputs: whole up to
+    DUMP_MAX_ELEMS elements, else its values at fixed seeded flat positions (a function of the element count only)."""
+    n = int(np.prod(x.shape))
+    idx = None if n <= DUMP_MAX_ELEMS else np.unique(np.random.default_rng(0).integers(0, n, DUMP_MAX_ELEMS))
+    if isinstance(x, np.ndarray):
+        return np.array(x if idx is None else x.ravel()[idx], dtype=np.float64)
+    import torch
+
+    flat = x.reshape(-1)
+    if idx is not None:
+        flat = flat[torch.from_numpy(idx).to(x.device)]
+    return flat.to(torch.float64).cpu().numpy().reshape(x.shape if idx is None else -1)
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ posterior + logpdf configs
 def run_infer(args, E, c):
     torch, blr, ctx = E.torch, E.blr, E.ctx
@@ -542,6 +571,10 @@ def run_infer(args, E, c):
         return post, lp
 
     ms_per_step, launches, clocks, (post, lp) = timed_steps(E, args, step)
+    if args.dump_outputs and E.rank == 0:
+        res = post.blr if rff is not None else post
+        write_dump(args.dump_outputs, {"posterior_mean": dump_sample(res.mw), "posterior_precision": dump_sample(res.Λw.dense()),
+                                       "logpdf": np.float64(lp)})
     gram_ms, solve_ms, prep_ms = gram_ms[-args.steps:], solve_ms[-args.steps:], prep_ms[-args.steps:]
     out = None
     if E.rank == 0:
@@ -661,8 +694,11 @@ def run_predict(args, E, c):
         ctx.check(ctx.lib.blr_rand_finite_dev(ctx.handle, dpost.handle, Xd.handle, C.byref(noise), S, None, None, 7 + E.rank,
                                               C.c_void_p(Y.data_ptr())))
 
+    dump = args.dump_outputs and E.rank == 0
     ms_mv, launches, clocks, _ = timed_steps(E, args, mean_var)
     ms_r, _, clocks_r, _ = timed_steps(E, args, rand)
+    if dump:  # Y is overwritten by rand_supplied below
+        outputs = {"mean": dump_sample(mv[0]), "var": dump_sample(mv[1]), "rand": dump_sample(Y)}
     # rand with SUPPLIED draws resident on the device -- the reference-parity mode (src/bayesian_linear_regression.jl:51-52: the
     # caller's RNG stream); the draws are generated once, outside the timed region (torch's generator: any N(0,1) stream will do)
     Zs = torch.randn((S, n), dtype=torch.float64, device="cuda", generator=torch.Generator(device="cuda").manual_seed(args.seed + 99))
@@ -673,6 +709,9 @@ def run_predict(args, E, c):
                                               7 + E.rank, C.c_void_p(Y.data_ptr())))
 
     ms_rs, _, clocks_rs, _ = timed_steps(E, args, rand_supplied)
+    if dump:
+        outputs["rand_supplied_draws"] = dump_sample(Y)
+        write_dump(args.dump_outputs, outputs)
     del Zs
     # parity on sampled blocks: x'm', |L^-1 x|² + σ² from the host posterior by torch (checker), rand with supplied draws
     Lp = np.linalg.cholesky(post.Λw.dense())
@@ -813,7 +852,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--scalar-noise", action="store_true", help="secondary measurement: Σy = σ² I instead of the headline's heteroscedastic noise")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float64; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

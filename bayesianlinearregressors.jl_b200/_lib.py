@@ -34,6 +34,13 @@ class Noise(C.Structure):
     _fields_ = [("kind", C.c_int), ("scalar", C.c_double), ("vec", C.c_void_p), ("dense", C.c_void_p), ("dense_ld", C.c_int64)]
 
 
+class LogpdfGrads(C.Structure):
+    """blr_logpdf_grads: NULL fields are not computed."""
+
+    _fields_ = [("dmw", c_double_p), ("dlambda", c_double_p), ("dsigma2", c_double_p), ("dsigma2_dev", C.c_void_p),
+                ("dy_dev", C.c_void_p), ("dX_dev", C.c_void_p), ("ld_dX", C.c_int64)]
+
+
 # name -> (restype, argtypes); every symbol include/blr_cuda.h declares (checked by tests/test_abi.py)
 SIGNATURES = {
     "blr_version": (C.c_int, []),
@@ -90,6 +97,8 @@ SIGNATURES = {
     ),
     "blr_logpdf_multi": (C.c_int, [C.c_void_p, C.POINTER(Prior), C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.POINTER(Noise),
                                   C.c_void_p]),
+    "blr_logpdf_grad": (C.c_int, [C.c_void_p, C.POINTER(Prior), C.c_void_p, C.c_void_p, C.POINTER(Noise), c_double_p,
+                                  C.POINTER(LogpdfGrads)]),
     "blr_infer": (
         C.c_int,
         [C.c_void_p, C.POINTER(Prior), C.c_void_p, C.c_void_p, C.POINTER(Noise), c_double_p, C.c_void_p, C.c_void_p,

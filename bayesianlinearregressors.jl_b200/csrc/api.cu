@@ -1009,6 +1009,96 @@ int blr_logpdf_multi(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const
     return done(0);
 }
 
+int blr_logpdf_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const blr_vec* y, const blr_noise* noise,
+                    double* logpdf_out, const blr_logpdf_grads* g) {
+    CTX_ENTER(ctx);
+    if (!prior || !x || !y || !noise || !prior->mw || !prior->lambda) return set_err(ctx, BLR_E_INVALID, "null argument");
+    if (prior->D > 0 && prior->D != x->D) return set_err(ctx, BLR_E_DIM, "size(X, 1) != length(mw)");
+    if (y->n != x->N) return set_err(ctx, BLR_E_DIM, "length(y) != size(fx.x.X, 2)");
+    if (noise->kind == BLR_NOISE_DENSE) return set_err(ctx, BLR_E_INVALID, "blr_logpdf_grad: dense Σy is not supported");
+    const blr_logpdf_grads none = {};
+    const blr_logpdf_grads& G = g ? *g : none;
+    const bool vector_noise = noise->kind == BLR_NOISE_VECTOR;
+    if ((G.dsigma2 && vector_noise) || (G.dsigma2_dev && !vector_noise))
+        return set_err(ctx, BLR_E_INVALID, "dsigma2 (scalar noise) / dsigma2_dev (vector noise) does not match the noise kind");
+    const int64_t D = x->D, N = x->N;
+    if (G.dX_dev && G.ld_dX < std::max<int64_t>(x->layout == BLR_COLVECS ? D : N, 1))
+        return set_err(ctx, BLR_E_INVALID, "ld_dX too small");
+    const double* sig = nullptr;
+    double sig_scalar = 0.0;
+    BLR_TRY(noise_args(ctx, noise, N, &sig, &sig_scalar, true));
+
+    // the value: exactly blr_infer's path (accumulate, all-reduce, infer_solve), keeping the posterior
+    blr_stats* s = nullptr;
+    blr_post* post = nullptr;
+    double* buf = nullptr;
+    BLR_TRY(blr_stats_create(ctx, D, &s));
+    auto done = [&](int rc) {
+        dev_free(ctx->stream, buf);
+        blr_stats_free(ctx, s);
+        if (post) post_release(post);
+        return rc;
+    };
+    int rc = blr_stats_accumulate(ctx, s, prior->mw, x, y, noise);
+    if (rc == 0) rc = blr_stats_allreduce(ctx, s);
+    if (rc == 0) rc = infer_solve(ctx, prior, s, logpdf_out, nullptr, nullptr, nullptr, &post);
+    if (rc == BLR_INFO_NOISE) {
+        int info = 1;
+        if (vector_noise && noise->vec) {
+            const int loc = check_noise_vector(ctx, noise->vec->p, noise->vec->n);
+            if (loc != 0) info = loc;
+        }
+        set_err(ctx, info, "observation noise variance is not positive");
+        return done(info);
+    }
+    if (rc != 0) return done(rc);
+
+    // device scratch: [se (N) | var (N) | Q (ldq x dk) | u (D) | mw (D) | λ (D) | dmw (D) | dλ (D or D x D) | Σ ∂/∂σ² (1)]
+    const bool obs = G.dX_dev || G.dy_dev || G.dsigma2_dev || G.dsigma2;
+    const bool diagonal = prior->lambda_kind == BLR_LAMBDA_DIAGONAL;
+    const bool needQ = G.dX_dev || (G.dlambda && !diagonal);
+    const bool fast = G.dX_dev && grad_x_fast_eligible(post, x, G.dX_dev, G.ld_dX);
+    int64_t ldq = 0, dk = 0;
+    if (needQ) grad_q_shape(post, fast, &ldq, &dk);
+    const int64_t nse = obs ? 2 * N : 0, nq = ldq * dk, ndl = diagonal ? D : D * D;
+    cudaError_t e = dev_alloc(ctx, &buf, (size_t)(nse + nq + 4 * D + ndl + 1) * sizeof(double));
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "cudaMallocAsync(logpdf_grad)"));
+    double *se = buf, *var = se + N, *Q = buf + nse, *u = Q + nq, *mwd = u + D, *lamd = mwd + D, *dmw = lamd + D, *dlam = dmw + D,
+           *dsum = dlam + ndl;
+    if (obs) {
+        rc = grad_obs(ctx, post, x, y->p, sig, sig_scalar, se, var, G.dy_dev, G.dsigma2_dev, G.dsigma2 ? dsum : nullptr);
+        if (rc == 0 && G.dsigma2 && ctx->nccl_comm && ctx->nranks > 1) {
+            NcclApi* a = nccl_api();
+            ncclResult_t r = a->AllReduce(dsum, dsum, 1, ncclFloat64, ncclSum, (ncclComm_t)ctx->nccl_comm, ctx->stream);
+            rc = (r != ncclSuccess) ? nccl_fail(ctx, r, "ncclAllReduce") : nccl_async_check(ctx);
+        }
+        if (rc != 0) return done(rc);
+    }
+    if (needQ) {
+        rc = grad_q(ctx, post, Q, ldq, dk);
+        if (rc != 0) return done(rc);
+    }
+    if (G.dmw || G.dlambda) {
+        e = cudaMemcpyAsync(mwd, prior->mw, (size_t)D * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess && diagonal)
+            e = cudaMemcpyAsync(lamd, prior->lambda, (size_t)D * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) return done(cuda_fail(ctx, e, "upload prior"));
+        rc = grad_prior(ctx, prior, post, mwd, diagonal ? lamd : nullptr, Q, ldq, u, G.dmw ? dmw : nullptr, G.dlambda ? dlam : nullptr);
+        if (rc != 0) return done(rc);
+    }
+    if (G.dX_dev) {
+        rc = grad_x(ctx, post, x, Q, ldq, dk, fast, se, sig, sig_scalar, G.dX_dev, G.ld_dX);
+        if (rc != 0) return done(rc);
+    }
+    if (G.dmw) e = cudaMemcpyAsync(G.dmw, dmw, (size_t)D * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && G.dlambda)
+        e = cudaMemcpyAsync(G.dlambda, dlam, (size_t)ndl * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && G.dsigma2) e = cudaMemcpyAsync(G.dsigma2, dsum, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "download logpdf gradients"));
+    return done(0);
+}
+
 // ---------------------------------------------------------------------------------------------- prediction
 int blr_post_create(blr_ctx* ctx, const blr_prior* prior, int64_t D, blr_post** out) {
     CTX_ENTER(ctx);

@@ -1,5 +1,6 @@
 // Internal declarations shared by the translation units of libblr_cuda.
 #pragma once
+#include <cuda.h>  // CUtensorMap (type only)
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -234,6 +235,25 @@ int sample_finite_fast(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, in
                        double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, const RandChunk* chunk = nullptr);
 int predict_mean_var_fast(blr_ctx* ctx, blr_post* p, const blr_x* x, const double* sigma2, double sigma2_scalar,
                           double* mean_dev, double* var_dev);
+// 2-D tiled TMA map of a column-major fp64 matrix (inner x outer, leading dimension ld), 128-byte swizzled boxes
+int make_tmap_2d_f64(blr_ctx* ctx, CUtensorMap* out, const double* base, uint64_t inner, uint64_t outer, uint64_t ld,
+                     uint32_t box_inner, uint32_t box_outer);
+
+// ---- grad.cu: gradients of the log marginal likelihood from the posterior p of the same call
+// e, h by the predict path with zero noise; on exit se = s ⊙ e; dy, dsig (N) and dsig_sum (device scalar) may be null
+int grad_obs(blr_ctx* ctx, blr_post* p, const blr_x* x, const double* y, const double* sigma2, double sigma2_scalar,
+             double* se, double* var, double* dy, double* dsig, double* dsig_sum);
+// u (D scratch) = m' - mw; dmw = Λw u; dlam = -1/2 (Q - Λw⁻¹ + u u') (dense, ld = D; Q read with leading dimension ldq) or its
+// diagonal (Q not read).  mw_dev, lam_dev (Diagonal prior only): the prior on the device; dmw / dlam may be null
+int grad_prior(blr_ctx* ctx, const blr_prior* prior, blr_post* p, const double* mw_dev, const double* lam_dev, const double* Q,
+               int64_t ldq, double* u, double* dmw, double* dlam);
+bool grad_x_fast_eligible(const blr_post* p, const blr_x* x, const double* dX, int64_t ld_dX);
+// shape of the Q buffer grad_x reads: zero-padded to the pass height and the stage depth of the fast kernel, else D x D
+void grad_q_shape(const blr_post* p, bool fast, int64_t* ldq, int64_t* dk);
+int grad_q(blr_ctx* ctx, blr_post* p, double* Qp, int64_t ldq, int64_t dk);
+// dX = -Q X S + m' se'  in x's layout
+int grad_x(blr_ctx* ctx, const blr_post* p, const blr_x* x, const double* Qp, int64_t ldq, int64_t dk, bool fast,
+           const double* se, const double* sigma2, double sigma2_scalar, double* dX, int64_t ld_dX);
 
 // ---- synth.cu
 int synth_normal(blr_ctx* ctx, double* out, int64_t rows, int64_t cols, int64_t ld, uint64_t seed, uint64_t stream_id,

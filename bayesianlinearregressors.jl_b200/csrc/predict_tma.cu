@@ -293,8 +293,8 @@ __global__ void pad_inverse_factor_kernel(const double* __restrict__ W, int D, d
 // `ld` elements apart, boxes of box_inner x box_outer elements stored with the 128-byte swizzle (box_inner * 8 <= 128 bytes),
 // out-of-range elements read as zero.  cuTensorMapEncodeTiled is a host-side encoder; it is looked up through the runtime
 // (cudaGetDriverEntryPoint) so the library keeps linking against nothing but cudart.
-static int make_tmap_2d_f64(blr_ctx* ctx, CUtensorMap* out, const double* base, uint64_t inner, uint64_t outer, uint64_t ld,
-                            uint32_t box_inner, uint32_t box_outer) {
+int make_tmap_2d_f64(blr_ctx* ctx, CUtensorMap* out, const double* base, uint64_t inner, uint64_t outer, uint64_t ld,
+                     uint32_t box_inner, uint32_t box_outer) {
     typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);

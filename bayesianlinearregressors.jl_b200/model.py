@@ -371,6 +371,147 @@ def _logpdf_multi(fx: FiniteGP, Y) -> np.ndarray:
     return out
 
 
+GRAD_KEYS = ("X", "y", "σ²", "mw", "Λw")
+
+
+def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatrix, yv: DeviceVector, Σy, wrt, out_like=None):
+    """One blr_logpdf_grad call.  Per-observation gradients are written into CUDA tensors on out_like's device when
+    `out_like` (a CUDA tensor) is given -- dX with the shape torch sees x in, (N, D) for ColVecs -- else downloaded into numpy
+    arrays (dX with the Julia-side shape).  Keys of `wrt` not in GRAD_KEYS are an error; keys left out get NULL."""
+    wrt = tuple(wrt)
+    bad = [k for k in wrt if k not in GRAD_KEYS]
+    if bad:
+        raise L.BLRError(L.E_INVALID, f"unknown gradient keys {bad}; expected a subset of {GRAD_KEYS}")
+    D = blr.mw.shape[0]
+    if X.D != D:  # `X' * mw` (:33) throws DimensionMismatch in the reference
+        raise L.DimensionMismatch(L.E_DIM, "size(X, 1) != length(mw)")
+    if yv.n != X.N:  # src/bayesian_linear_regression.jl:74
+        raise L.DimensionMismatch(L.E_DIM, "length(y) != size(fx.x.X, 2)")
+    noise, keep_noise = make_noise(ctx, Σy, X.N)
+    prior, keep_prior = blr._prior_struct()
+    N, colv = X.N, X.layout == L.COLVECS
+    vector_noise = noise.kind == L.NOISE_VECTOR
+    g = L.LogpdfGrads()
+    out, dev = {}, {}
+    if "mw" in wrt:
+        out["mw"] = np.empty(D)
+        g.dmw = out["mw"].ctypes.data_as(L.c_double_p)
+    if "Λw" in wrt:
+        out["Λw"] = np.empty(D) if isinstance(blr.Λw, Diagonal) else np.empty((D, D), order="F")
+        g.dlambda = out["Λw"].ctypes.data_as(L.c_double_p)
+    dσ2_host = C.c_double()
+    if "σ²" in wrt and not vector_noise:
+        g.dsigma2 = C.pointer(dσ2_host)
+    if out_like is not None:
+        import torch
+
+        def buf(*shape):
+            return torch.empty(shape, dtype=torch.float64, device=out_like.device)
+    else:
+        def buf(*shape):
+            return DeviceVector.alloc(ctx, int(np.prod(shape)))
+
+    def addr(b):
+        return b.data_ptr() if out_like is not None else b.device_ptr()
+
+    if "y" in wrt:
+        dev["y"] = buf(N)
+        g.dy_dev = addr(dev["y"])
+    if "σ²" in wrt and vector_noise:
+        dev["σ²"] = buf(N)
+        g.dsigma2_dev = addr(dev["σ²"])
+    if "X" in wrt:
+        dev["X"] = buf(N, D) if colv else buf(D, N)  # torch row-major (N, D) == column-major D x N (ColVecs); (D, N) for RowVecs
+        g.dX_dev = addr(dev["X"])
+        g.ld_dX = max(D if colv else N, 1)
+    if out_like is not None:  # the output tensors were just allocated on torch's stream
+        ctx.wait_torch_stream(out_like)
+    lp = C.c_double()
+    ctx.check(ctx.lib.blr_logpdf_grad(ctx.handle, C.byref(prior), X.handle, yv.handle, C.byref(noise), C.byref(lp), C.byref(g)))
+    if "σ²" in wrt and not vector_noise:
+        out["σ²"] = dσ2_host.value
+    if out_like is not None:
+        ctx.release_to_torch_stream(out_like.device)
+        out.update(dev)
+    else:
+        for k, v in dev.items():
+            a = v.download()
+            out[k] = a.reshape((D, N) if colv else (N, D), order="F") if k == "X" else a
+    return lp.value, out
+
+
+def logpdf_and_grad(fx: FiniteGP, y, wrt=GRAD_KEYS):
+    """logpdf(fx, y) and its gradients with respect to the keys of `wrt` -- "X" (the inputs; ϕ(x) for a BasisFunctionRegressor),
+    "y", "σ²" (a scalar for scalar noise, else one per observation), "mw" and "Λw" (D values for a Diagonal prior, else the
+    symmetric D x D G with dℓ = <G, dΛw>) -- in closed form on the device (blr_logpdf_grad).  Returns (logpdf, dict).
+    Per-observation gradients of inputs given as CUDA tensors come back as CUDA tensors (dX with x's tensor shape, (N, D) for
+    ColVecs); otherwise everything is numpy (dX D x N for ColVecs, N x D for RowVecs)."""
+    fx = _to_finite_blr(fx)
+    ctx = fx._context()
+    X = x_as_colvecs(ctx, fx.x)
+    yv = _as_device_vector(ctx, y)
+    out_like = None
+    for cand in (fx.x.X, y):
+        if _is_torch_cuda(cand):
+            out_like = cand
+            break
+    return _logpdf_grad_call(ctx, fx.f, X, yv, fx.Σy, wrt, out_like)
+
+
+def _torch_logpdf_function():
+    import torch
+
+    class TorchLogpdf(torch.autograd.Function):
+        """ℓ(X, y, mw, Λw, σ²) as a differentiable torch op; forward computes the gradients the backward needs in the same call
+        (blr_logpdf_grad), backward only scales them by grad_output."""
+
+        @staticmethod
+        def forward(fctx, X, y, mw, Λw, σ2):
+            ctx = default_context()
+            if not (X.is_cuda and X.dtype == torch.float64 and X.dim() == 2):
+                raise L.BLRError(L.E_INVALID, "torch_logpdf: X must be an (N, D) float64 CUDA tensor")
+            mw_h = mw.detach().to("cpu", torch.float64).numpy()
+            lam_h = Λw.detach().to("cpu", torch.float64).numpy()
+            blr = BayesianLinearRegressor(mw_h, Diagonal(lam_h) if lam_h.ndim == 1 else lam_h)
+            Xc = X.detach().contiguous()
+            Xd = DeviceMatrix.wrap_torch(ctx, Xc, L.COLVECS)
+            yv = DeviceVector.wrap_torch(ctx, y.detach().to(torch.float64).contiguous())
+            Σy = float(σ2) if σ2.dim() == 0 else σ2.detach().to(torch.float64).contiguous()
+            need = fctx.needs_input_grad
+            wrt = [k for k, n in zip(GRAD_KEYS, (need[0], need[1], need[4], need[2], need[3])) if n]
+            lp, g = _logpdf_grad_call(ctx, blr, Xd, yv, Σy, wrt, out_like=Xc)
+            grads = []
+            for k, like in (("X", X), ("y", y), ("mw", mw), ("Λw", Λw), ("σ²", σ2)):
+                v = g.get(k)
+                if v is not None and not isinstance(v, torch.Tensor):
+                    v = torch.as_tensor(np.asarray(v), dtype=torch.float64, device=like.device).reshape(like.shape)
+                grads.append(v)
+            fctx.save_for_backward(*[v if v is not None else torch.empty(0) for v in grads])
+            fctx.present = [v is not None for v in grads]
+            return torch.tensor(lp, dtype=torch.float64, device=X.device)
+
+        @staticmethod
+        def backward(fctx, grad_out):
+            saved = fctx.saved_tensors
+            return tuple(grad_out * v if present else None for v, present in zip(saved, fctx.present))
+
+    return TorchLogpdf
+
+
+_TORCH_LOGPDF = None
+
+
+def torch_logpdf(X, y, mw, Λw, σ2):
+    """Differentiable logpdf of y under BayesianLinearRegressor(mw, Λw)(ColVecs(X), σ²) for float64 CUDA tensors: X is (N, D),
+    Λw is (D,) (Diagonal prior) or (D, D), σ² is 0-d (scalar noise) or (N,).  The gradients of the inputs that require them are
+    computed on the device in the forward call; this is what makes a TorchFeatureMap's network trainable by type-II maximum
+    likelihood (the reference's examples/nn-blr.jl)."""
+    global _TORCH_LOGPDF
+    if _TORCH_LOGPDF is None:
+        _TORCH_LOGPDF = _torch_logpdf_function()
+    return _TORCH_LOGPDF.apply(X, y, mw, Λw, σ2)
+
+
 def posterior(fx: FiniteGP, y):
     """src/bayesian_linear_regression.jl:60-69 / basis_function_regression.jl:62-65."""
     post = _infer(fx, y, False, True)[1]

@@ -161,7 +161,7 @@ int blr_x_features(blr_ctx* ctx, const blr_x* xin, const double* W, const double
 
 /* ------------------------------------------------------------------ inference
  * replaces __compute_inference_quantities / logpdf / posterior,
- * src/bayesian_linear_regression.jl:55-89 */
+ * src/bayesian_linear_regression.jl:55-89, and the reverse-mode derivative of logpdf (blr_logpdf_grad) */
 int blr_stats_create(blr_ctx* ctx, int64_t D, blr_stats** out);
 int blr_stats_free(blr_ctx* ctx, blr_stats* s);
 int blr_stats_zero(blr_ctx* ctx, blr_stats* s);
@@ -203,6 +203,26 @@ int blr_infer(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const blr_ve
  * Scalar / vector Σy only (dense Σy: BLR_E_INVALID -- loop blr_infer).  Statistics are all-reduced when a communicator is set. */
 int blr_logpdf_multi(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const double* Y_dev, int64_t ldy, int64_t k,
                      const blr_noise* noise, double* logpdf_out);
+/* Gradients of the log marginal likelihood (:55-58) with respect to every input, in closed form from the posterior of the same
+ * call (type-II maximum likelihood of mw, Λw, Σy, and backpropagation into whatever produced X or y).  With s_n = 1/σ²_n,
+ * Q = inverse posterior precision, m' the posterior mean, u = m' - mw and e_n = y_n - x_n'm':
+ *   ∂/∂x_n = s_n (e_n m' - Q x_n)    ∂/∂y_n = -s_n e_n    ∂/∂σ²_n = (s_n² (x_n'Q x_n + e_n²) - s_n) / 2
+ *   ∂/∂mw  = Λw u                    ∂/∂Λw  = -(Q - Λw⁻¹ + u u') / 2  (the symmetric G with dℓ = <G, dΛw>; its diagonal for
+ *                                                                      a Diagonal prior)
+ * Any field may be NULL (not computed); a pass over the observations runs only when a per-observation output or the scalar
+ * dsigma2 is requested.  logpdf_out (may be NULL) is bit-identical to blr_infer's.  Scalar / vector Σy only (dense Σy:
+ * BLR_E_INVALID).  Per-observation outputs cover this rank's shard; the others are replicated on every rank. */
+typedef struct blr_logpdf_grads {
+    double* dmw;         /* host, D */
+    double* dlambda;     /* host: D (BLR_LAMBDA_DIAGONAL) or D x D column-major, ld = D (BLR_LAMBDA_DENSE) */
+    double* dsigma2;     /* host, 1 value: BLR_NOISE_SCALAR (summed over all ranks) */
+    double* dsigma2_dev; /* device, N: BLR_NOISE_VECTOR (this rank's shard) */
+    double* dy_dev;      /* device, N (this rank's shard) */
+    double* dX_dev;      /* device, same layout as x (this rank's shard) */
+    int64_t ld_dX;       /* >= D (COLVECS) or >= N (ROWVECS) */
+} blr_logpdf_grads;
+int blr_logpdf_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const blr_vec* y, const blr_noise* noise,
+                    double* logpdf_out, const blr_logpdf_grads* g);
 
 /* ------------------------------------------------------------------ prediction / sampling
  * replaces mean / var / mean_and_var / rand, src/bayesian_linear_regression.jl:33-53,

@@ -2,6 +2,7 @@
 # The struct, the FiniteBLR alias, x_as_colvecs and every signature are unchanged; only the bodies dispatch to
 # libblr_cuda.  UNEXECUTED (no Julia in the build image) -- see INTEGRATION.md.
 using .LibBLR: LibBLR
+using ChainRulesCore: ChainRulesCore      # a dependency of AbstractGPs
 
 # layout + device upload of whatever x_as_colvecs accepts (:20-31); errors for unknown vectors are preserved.
 _device_x(ctx, x::ColVecs) = LibBLR.upload_x(ctx, x.X, LibBLR.COLVECS)
@@ -73,6 +74,33 @@ function AbstractGPs.logpdf(fx::FiniteBLR, Y::AbstractMatrix{<:Real})
     prior, keep1 = _prior(fx.f)
     noise, keep2 = _noise(ctx, fx.Σy)
     GC.@preserve keep1 keep2 x LibBLR.logpdf_multi(ctx, prior, x, Matrix{Float64}(Y), noise)
+end
+
+# Reverse-mode rule for logpdf (:55-58): Zygote cannot enter the ccall above, so the gradients come in closed form from the
+# device (blr_logpdf_grad, one call for the value and every tangent).  Tangents for fx.f.mw, fx.f.Λw (the diagonal of a
+# Diagonal, else the symmetric D x D G with dℓ = <G, dΛw>), fx.x.X (ColVecs or RowVecs), fx.Σy (Diagonal(Fill) or Diagonal)
+# and y.  Dense Σy has no rule (the library returns an error).
+function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteBLR, y::AbstractVector{<:Real})
+    ctx = LibBLR.default_context()
+    length(y) == length(fx.x) || throw(error("length(y) != size(fx.x.X, 2)"))            # :74
+    prior, keep1 = _prior(fx.f)
+    x = _device_x(ctx, fx.x)
+    yv = LibBLR.upload_vec(ctx, collect(Float64, y))
+    noise, keep2 = _noise(ctx, fx.Σy)
+    layout = fx.x isa ColVecs ? LibBLR.COLVECS : LibBLR.ROWVECS
+    lp, dX, dy, dσ², dmw, dΛ = GC.@preserve keep1 keep2 x yv LibBLR.logpdf_grad(ctx, prior, x, layout, yv, noise;
+                                                                                  diagonal=fx.f.Λw isa Diagonal)
+    function logpdf_pullback(Δ)
+        Δ = ChainRulesCore.unthunk(Δ)
+        Λ̄ = fx.f.Λw isa Diagonal ? ChainRulesCore.Tangent{typeof(fx.f.Λw)}(diag=Δ .* dΛ) : Δ .* dΛ
+        Σ̄ = fx.Σy isa Diagonal{<:Real,<:FillArrays.Fill} ?
+            ChainRulesCore.Tangent{typeof(fx.Σy)}(diag=ChainRulesCore.Tangent{typeof(fx.Σy.diag)}(value=Δ * dσ²)) :
+            ChainRulesCore.Tangent{typeof(fx.Σy)}(diag=Δ .* dσ²)
+        f̄ = ChainRulesCore.Tangent{typeof(fx.f)}(mw=Δ .* dmw, Λw=Λ̄)
+        x̄ = ChainRulesCore.Tangent{typeof(fx.x)}(X=Δ .* dX)
+        return ChainRulesCore.NoTangent(), ChainRulesCore.Tangent{typeof(fx)}(f=f̄, x=x̄, Σy=Σ̄), Δ .* dy
+    end
+    return lp, logpdf_pullback
 end
 
 function AbstractGPs.posterior(fx::FiniteBLR, y::AbstractVector{<:Real})                           # :60-69

@@ -138,6 +138,53 @@ function logpdf_multi(ctx::Context, prior::Prior, x::DeviceX, Y::Matrix{Float64}
     return out
 end
 
+# gradients of logpdf (blr_logpdf_grad): the per-observation ones land in library-owned device vectors and are downloaded;
+# returns (logpdf, dX (shaped like the input matrix), dy, dσ² (a number for scalar noise), dmw, dΛw (vector for a Diagonal prior))
+struct LogpdfGrads
+    dmw::Ptr{Float64}
+    dlambda::Ptr{Float64}
+    dsigma2::Ptr{Float64}       # host, scalar noise
+    dsigma2_dev::Ptr{Float64}   # device, vector noise
+    dy_dev::Ptr{Float64}
+    dX_dev::Ptr{Float64}
+    ld_dX::Int64
+end
+function _alloc_vec(ctx::Context, n::Integer)
+    r = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ctx, ccall((:blr_vec_alloc, libblr), Cint, (Ptr{Cvoid}, Int64, Ref{Ptr{Cvoid}}), ctx.ptr, n, r))
+    h = DeviceVec(r[], ctx)
+    finalizer(h -> ccall((:blr_vec_free, libblr), Cint, (Ptr{Cvoid}, Ptr{Cvoid}), h.ctx.ptr, h.ptr), h)
+    p = Ref{Ptr{Float64}}(C_NULL)
+    check(ctx, ccall((:blr_vec_device_ptr, libblr), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ref{Ptr{Float64}}), ctx.ptr, h.ptr, p))
+    return h, p[]
+end
+function _download(ctx::Context, h::DeviceVec, n::Integer)
+    out = Vector{Float64}(undef, n)
+    check(ctx, ccall((:blr_vec_download, libblr), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}), ctx.ptr, h.ptr, out))
+    return out
+end
+function logpdf_grad(ctx::Context, prior::Prior, x::DeviceX, layout::Cint, y::DeviceVec, noise::Noise; diagonal::Bool)
+    D, N = x.D, x.N
+    dmw = Vector{Float64}(undef, D)
+    dΛ = diagonal ? Vector{Float64}(undef, D) : Matrix{Float64}(undef, D, D)
+    dσ²_host = Ref{Float64}(NaN)
+    vector_noise = noise.kind == NOISE_VECTOR
+    hX, pX = _alloc_vec(ctx, D * N)
+    hy, py = _alloc_vec(ctx, N)
+    hs, ps = vector_noise ? _alloc_vec(ctx, N) : (nothing, Ptr{Float64}(C_NULL))
+    lp = Ref{Float64}(NaN)
+    GC.@preserve dmw dΛ dσ²_host begin
+        g = LogpdfGrads(pointer(dmw), pointer(dΛ), vector_noise ? C_NULL : Base.unsafe_convert(Ptr{Float64}, dσ²_host), ps, py, pX,
+                        max(layout == COLVECS ? D : N, 1))
+        check(ctx, ccall((:blr_logpdf_grad, libblr), Cint,
+            (Ptr{Cvoid}, Ref{Prior}, Ptr{Cvoid}, Ptr{Cvoid}, Ref{Noise}, Ref{Float64}, Ref{LogpdfGrads}),
+            ctx.ptr, prior, x.ptr, y.ptr, noise, lp, g))
+    end
+    dX = reshape(_download(ctx, hX, D * N), layout == COLVECS ? (D, N) : (N, D))
+    dσ² = vector_noise ? _download(ctx, hs, N) : dσ²_host[]
+    return lp[], dX, _download(ctx, hy, N), dσ², dmw, dΛ
+end
+
 # the same from host arrays: blr_stats_create -> blr_stats_accumulate_host -> blr_stats_allreduce -> blr_infer_from_stats
 function infer_host(ctx::Context, prior::Prior, X::StridedMatrix{Float64}, layout::Cint, y::Vector{Float64}, Σy;
                     want_T::Bool=false, chunk::Integer=1 << 16)

@@ -99,6 +99,8 @@ SIGNATURES = {
                                   C.c_void_p]),
     "blr_logpdf_grad": (C.c_int, [C.c_void_p, C.POINTER(Prior), C.c_void_p, C.c_void_p, C.POINTER(Noise), c_double_p,
                                   C.POINTER(LogpdfGrads)]),
+    "blr_logpdf_multi_grad": (C.c_int, [C.c_void_p, C.POINTER(Prior), C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
+                                        C.POINTER(Noise), c_double_p, c_double_p, C.POINTER(LogpdfGrads)]),
     "blr_infer": (
         C.c_int,
         [C.c_void_p, C.POINTER(Prior), C.c_void_p, C.c_void_p, C.POINTER(Noise), c_double_p, C.c_void_p, C.c_void_p,

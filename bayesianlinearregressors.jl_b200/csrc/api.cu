@@ -927,6 +927,77 @@ int blr_infer(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const blr_ve
     return rc;
 }
 
+// The body of logpdf(fx, Y::AbstractMatrix) shared by blr_logpdf_multi and blr_logpdf_multi_grad (arguments validated, k >= 1):
+// accumulate column 0, R = X Σy⁻¹ (Y_j - X'mw) of columns 1 .. k-1, all-reduce, infer_solve, Z_j = L⁻¹ R_j in place.  On
+// return the caller owns *s (the reduced statistics), *post (the posterior of column 0) and *extra = [Z (K x D) | q (K) | zz (K) |
+// q_0 | z_0'z_0] (K = k - 1; null when K = 0), whatever the status; logpdf_out (host, k) is filled on success.
+static int logpdf_multi_forward(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const double* Y_dev, int64_t ldy, int64_t k,
+                                const blr_noise* noise, double* logpdf_out, blr_stats** s_out, blr_post** post_out,
+                                double** extra_out) {
+    const int64_t D = x->D, N = x->N, K = k - 1;
+    blr_vec y0;  // column 0 goes down the ordinary path: Gram statistics, factorisation, logpdf_0
+    y0.p = const_cast<double*>(Y_dev);
+    y0.n = N;
+    BLR_TRY(blr_stats_create(ctx, D, s_out));
+    blr_stats* s = *s_out;
+    int rc = blr_stats_accumulate(ctx, s, prior->mw, x, &y0, noise);
+    if (rc != 0) return rc;
+    if (K > 0) {
+        cudaError_t e = dev_alloc(ctx, extra_out, (size_t)(K * D + 2 * K + 2) * sizeof(double));
+        if (e != cudaSuccess) return cuda_fail(ctx, e, "cudaMallocAsync(logpdf_multi)");
+        const double* sig = nullptr;
+        double sig_scalar = 0.0;
+        rc = noise_args(ctx, noise, N, &sig, &sig_scalar, true);
+        if (rc != 0) return rc;
+        bool zero = true;
+        for (int64_t i = 0; i < D; ++i)
+            if (prior->mw[i] != 0.0) zero = false;
+        double* pm = nullptr;  // X'mw, shared by every column
+        if (!zero && N > 0) {
+            e = dev_alloc(ctx, &pm, (size_t)N * sizeof(double));
+            if (e != cudaSuccess) return cuda_fail(ctx, e, "cudaMallocAsync(pm)");
+            // blr_stats_accumulate left mw in ctx->small + SMALL_MW (stream-ordered)
+            rc = apply_weights(ctx, x, ctx->small + SMALL_MW, pm);
+        }
+        if (rc == 0) rc = rhs_multi(ctx, x, Y_dev + ldy, ldy, K, sig, sig_scalar, pm, *extra_out, *extra_out + K * D);
+        dev_free(ctx->stream, pm);
+        if (rc != 0) return rc;
+    }
+    double* extra = *extra_out;
+    rc = blr_stats_allreduce(ctx, s);
+    if (rc == 0 && K > 0 && ctx->nccl_comm && ctx->nranks > 1) {
+        NcclApi* a = nccl_api();
+        ncclResult_t r = a->AllReduce(extra, extra, (size_t)(K * D + K), ncclFloat64, ncclSum, (ncclComm_t)ctx->nccl_comm, ctx->stream);
+        rc = (r != ncclSuccess) ? nccl_fail(ctx, r, "ncclAllReduce") : nccl_async_check(ctx);
+    }
+    if (rc != 0) return rc;
+    rc = infer_solve(ctx, prior, s, logpdf_out, nullptr, nullptr, nullptr, post_out);
+    if (rc == BLR_INFO_NOISE) {
+        int info = 1;
+        if (noise && noise->kind == BLR_NOISE_VECTOR && noise->vec) {
+            const int loc = check_noise_vector(ctx, noise->vec->p, noise->vec->n);
+            if (loc != 0) info = loc;
+        }
+        set_err(ctx, info, "observation noise variance is not positive");
+        return info;
+    }
+    if (rc != 0 || K == 0) return rc;
+    // logpdf_j - logpdf_0 = -1/2 [(q_j - q_0) - (z_j'z_j - z_0'z_0)]: every other term of (:57) is common to the columns
+    double* tail = extra + K * D;
+    BLR_TRY(forward_solve_multi(ctx, *post_out, extra, K, tail + K));
+    std::vector<double> h((size_t)(2 * K + 2));
+    cudaError_t e = cudaMemcpyAsync(tail + 2 * K, s->scal(), sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(tail + 2 * K + 1, ctx->small + SMALL_SC + 2, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(h.data(), tail, h.size() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "download logpdf_multi");
+    const double q0 = h[2 * K], zz0 = h[2 * K + 1];
+    for (int64_t j = 0; j < K; ++j) logpdf_out[j + 1] = logpdf_out[0] - 0.5 * ((h[j] - q0) - (h[K + j] - zz0));
+    return 0;
+}
+
 int blr_logpdf_multi(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const double* Y_dev, int64_t ldy, int64_t k,
                      const blr_noise* noise, double* logpdf_out) {
     CTX_ENTER(ctx);
@@ -937,76 +1008,14 @@ int blr_logpdf_multi(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const
     if (ldy < x->N) return set_err(ctx, BLR_E_DIM, "size(Y, 1) != size(fx.x.X, 2)");
     if (noise && noise->kind == BLR_NOISE_DENSE)
         return set_err(ctx, BLR_E_INVALID, "blr_logpdf_multi: dense Σy is not supported (loop blr_infer over the columns)");
-    const int64_t D = x->D, N = x->N, K = k - 1;
-    blr_vec y0;  // column 0 goes down the ordinary path: Gram statistics, factorisation, logpdf_0
-    y0.p = const_cast<double*>(Y_dev);
-    y0.n = N;
     blr_stats* s = nullptr;
     blr_post* post = nullptr;
-    double* extra = nullptr;  // [R (K x D) | q (K) | zz (K) | q_0 | z_0'z_0]
-    BLR_TRY(blr_stats_create(ctx, D, &s));
-    auto done = [&](int rc) {
-        dev_free(ctx->stream, extra);
-        blr_stats_free(ctx, s);
-        if (post) post_release(post);
-        return rc;
-    };
-    int rc = blr_stats_accumulate(ctx, s, prior->mw, x, &y0, noise);
-    if (rc != 0) return done(rc);
-    if (K > 0) {
-        cudaError_t e = dev_alloc(ctx, &extra, (size_t)(K * D + 2 * K + 2) * sizeof(double));
-        if (e != cudaSuccess) return done(cuda_fail(ctx, e, "cudaMallocAsync(logpdf_multi)"));
-        const double* sig = nullptr;
-        double sig_scalar = 0.0;
-        rc = noise_args(ctx, noise, N, &sig, &sig_scalar, true);
-        if (rc != 0) return done(rc);
-        bool zero = true;
-        for (int64_t i = 0; i < D; ++i)
-            if (prior->mw[i] != 0.0) zero = false;
-        double* pm = nullptr;  // X'mw, shared by every column
-        if (!zero && N > 0) {
-            e = dev_alloc(ctx, &pm, (size_t)N * sizeof(double));
-            if (e != cudaSuccess) return done(cuda_fail(ctx, e, "cudaMallocAsync(pm)"));
-            // blr_stats_accumulate left mw in ctx->small + SMALL_MW (stream-ordered)
-            rc = apply_weights(ctx, x, ctx->small + SMALL_MW, pm);
-        }
-        if (rc == 0) rc = rhs_multi(ctx, x, Y_dev + ldy, ldy, K, sig, sig_scalar, pm, extra, extra + K * D);
-        dev_free(ctx->stream, pm);
-        if (rc != 0) return done(rc);
-    }
-    rc = blr_stats_allreduce(ctx, s);
-    if (rc == 0 && K > 0 && ctx->nccl_comm && ctx->nranks > 1) {
-        NcclApi* a = nccl_api();
-        ncclResult_t r = a->AllReduce(extra, extra, (size_t)(K * D + K), ncclFloat64, ncclSum, (ncclComm_t)ctx->nccl_comm, ctx->stream);
-        rc = (r != ncclSuccess) ? nccl_fail(ctx, r, "ncclAllReduce") : nccl_async_check(ctx);
-    }
-    if (rc != 0) return done(rc);
-    rc = infer_solve(ctx, prior, s, logpdf_out, nullptr, nullptr, nullptr, &post);
-    if (rc == BLR_INFO_NOISE) {
-        int info = 1;
-        if (noise && noise->kind == BLR_NOISE_VECTOR && noise->vec) {
-            const int loc = check_noise_vector(ctx, noise->vec->p, noise->vec->n);
-            if (loc != 0) info = loc;
-        }
-        set_err(ctx, info, "observation noise variance is not positive");
-        return done(info);
-    }
-    if (rc != 0 || K == 0) return done(rc);
-    // logpdf_j - logpdf_0 = -1/2 [(q_j - q_0) - (z_j'z_j - z_0'z_0)]: every other term of (:57) is common to the columns
-    double* tail = extra + K * D;
-    rc = forward_solve_multi(ctx, post, extra, K, tail + K);
-    if (rc != 0) return done(rc);
-    std::vector<double> h((size_t)(2 * K + 2));
-    cudaError_t e = cudaMemcpyAsync(tail + 2 * K, s->scal(), sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(tail + 2 * K + 1, ctx->small + SMALL_SC + 2, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(h.data(), tail, h.size() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "download logpdf_multi"));
-    const double q0 = h[2 * K], zz0 = h[2 * K + 1];
-    for (int64_t j = 0; j < K; ++j) logpdf_out[j + 1] = logpdf_out[0] - 0.5 * ((h[j] - q0) - (h[K + j] - zz0));
-    return done(0);
+    double* extra = nullptr;
+    const int rc = logpdf_multi_forward(ctx, prior, x, Y_dev, ldy, k, noise, logpdf_out, &s, &post, &extra);
+    dev_free(ctx->stream, extra);
+    if (s) blr_stats_free(ctx, s);
+    if (post) post_release(post);
+    return rc;
 }
 
 int blr_logpdf_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const blr_vec* y, const blr_noise* noise,
@@ -1090,6 +1099,113 @@ int blr_logpdf_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const 
         rc = grad_x(ctx, post, x, Q, ldq, dk, fast, se, sig, sig_scalar, G.dX_dev, G.ld_dX);
         if (rc != 0) return done(rc);
     }
+    if (G.dmw) e = cudaMemcpyAsync(G.dmw, dmw, (size_t)D * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && G.dlambda)
+        e = cudaMemcpyAsync(G.dlambda, dlam, (size_t)ndl * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && G.dsigma2) e = cudaMemcpyAsync(G.dsigma2, dsum, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "download logpdf gradients"));
+    return done(0);
+}
+
+int blr_logpdf_multi_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const double* Y_dev, int64_t ldy, int64_t k,
+                          const blr_noise* noise, const double* weights, double* logpdf_out, const blr_logpdf_grads* g) {
+    CTX_ENTER(ctx);
+    if (!prior || !x || !noise || !prior->mw || !prior->lambda || k < 0 || (k > 0 && !Y_dev))
+        return set_err(ctx, BLR_E_INVALID, "null argument");
+    if (prior->D > 0 && prior->D != x->D) return set_err(ctx, BLR_E_DIM, "size(X, 1) != length(mw)");
+    if (k > 0 && ldy < x->N) return set_err(ctx, BLR_E_DIM, "size(Y, 1) != size(fx.x.X, 2)");
+    if (noise->kind == BLR_NOISE_DENSE) return set_err(ctx, BLR_E_INVALID, "blr_logpdf_multi_grad: dense Σy is not supported");
+    const blr_logpdf_grads none = {};
+    const blr_logpdf_grads& G = g ? *g : none;
+    const bool vector_noise = noise->kind == BLR_NOISE_VECTOR;
+    if ((G.dsigma2 && vector_noise) || (G.dsigma2_dev && !vector_noise))
+        return set_err(ctx, BLR_E_INVALID, "dsigma2 (scalar noise) / dsigma2_dev (vector noise) does not match the noise kind");
+    const int64_t D = x->D, N = x->N;
+    const bool colv = x->layout == BLR_COLVECS;
+    if (G.dX_dev && G.ld_dX < std::max<int64_t>(colv ? D : N, 1)) return set_err(ctx, BLR_E_INVALID, "ld_dX too small");
+    const bool diagonal = prior->lambda_kind == BLR_LAMBDA_DIAGONAL;
+    const int64_t ndl = diagonal ? D : D * D;
+    if (k == 0) {  // L is an empty sum: every requested gradient is zero
+        cudaStream_t sm = ctx->stream;
+        if (G.dmw) std::fill(G.dmw, G.dmw + D, 0.0);
+        if (G.dlambda) std::fill(G.dlambda, G.dlambda + ndl, 0.0);
+        if (G.dsigma2) *G.dsigma2 = 0.0;
+        if (G.dsigma2_dev && N > 0) BLR_CUDA_OK(ctx, cudaMemsetAsync(G.dsigma2_dev, 0, (size_t)N * sizeof(double), sm));
+        if (G.dX_dev && N > 0 && D > 0) {
+            const int64_t rows = colv ? D : N, cols = colv ? N : D;
+            BLR_CUDA_OK(ctx, cudaMemset2DAsync(G.dX_dev, (size_t)G.ld_dX * sizeof(double), 0, (size_t)rows * sizeof(double), (size_t)cols, sm));
+        }
+        BLR_CUDA_OK(ctx, cudaStreamSynchronize(sm));
+        return 0;
+    }
+    const double* sig = nullptr;
+    double sig_scalar = 0.0;
+    BLR_TRY(noise_args(ctx, noise, N, &sig, &sig_scalar, true));
+    std::vector<double> c_host(weights ? weights : nullptr, weights ? weights + k : nullptr), lp_host;
+    if (!weights) c_host.assign((size_t)k, 1.0);
+    double cbar = 0.0;
+    for (int64_t j = 0; j < k; ++j) cbar += c_host[j];
+    if (!logpdf_out) {
+        lp_host.resize((size_t)k);
+        logpdf_out = lp_host.data();
+    }
+
+    // the value: exactly blr_logpdf_multi's path, keeping the posterior of column 0 and Z = L⁻¹R of the others
+    blr_stats* s = nullptr;
+    blr_post* post = nullptr;
+    double *extra = nullptr, *buf = nullptr;
+    auto done = [&](int rc) {
+        dev_free(ctx->stream, buf);
+        dev_free(ctx->stream, extra);
+        if (s) blr_stats_free(ctx, s);
+        if (post) post_release(post);
+        return rc;
+    };
+    int rc = logpdf_multi_forward(ctx, prior, x, Y_dev, ldy, k, noise, logpdf_out, &s, &post, &extra);
+    if (rc != 0) return done(rc);
+
+    // device scratch: [A (ldq x (dk + kp)) | E (kp x N) | c (k) | U (D x k) | M' (D x k) | uc (D) | mw (D) | λ (D) | dmw (D) |
+    //                  dλ (D or D x D) | Σ ∂/∂σ² (1) | XM (N x k) | mean, h (2N)]: A and E first, where the tensor copies need
+    //                  16-byte alignment (ldq and kp are multiples of 16 on the fast path)
+    const bool obs = G.dX_dev || G.dy_dev || G.dsigma2_dev || G.dsigma2;
+    const bool wsig = G.dsigma2_dev || G.dsigma2;
+    const bool needQ = G.dX_dev || (G.dlambda && !diagonal);
+    const bool fast = G.dX_dev && grad_x_fast_eligible(post, x, G.dX_dev, G.ld_dX);
+    const int64_t kp = (k + 15) / 16 * 16;
+    int64_t ldq = 0, dk = 0;
+    if (needQ) grad_q_shape(post, fast, &ldq, &dk);
+    const int64_t nsmall = k + 2 * D * k + 5 * D + ndl + 1, nxm = obs ? N * k : 0, nh = wsig ? 2 * N : 0,
+                  ne = G.dX_dev ? kp * N : 0, na = needQ ? ldq * (dk + (G.dX_dev ? kp : 0)) : 0;
+    cudaError_t e = dev_alloc(ctx, &buf, (size_t)(nsmall + nxm + nh + ne + na) * sizeof(double));
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "cudaMallocAsync(logpdf_multi_grad)"));
+    double *A = buf, *E = A + na, *c = E + ne, *U = c + k, *M = U + D * k, *uc = M + D * k, *mwd = uc + D, *lamd = mwd + D,
+           *dmw = lamd + D, *dlam = dmw + D, *dsum = dlam + ndl, *XM = dsum + 1, *hbuf = XM + nxm;
+    e = cudaMemcpyAsync(c, c_host.data(), (size_t)k * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(mwd, prior->mw, (size_t)D * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && diagonal)
+        e = cudaMemcpyAsync(lamd, prior->lambda, (size_t)D * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "upload weights / prior"));
+    // U and M' are replicated: R, hence Z, was all-reduced by the forward pass
+    rc = grad_means_multi(ctx, post, mwd, extra, k, U, M);
+    if (rc == 0 && obs) {
+        rc = grad_obs_multi(ctx, post, x, M, k, kp, Y_dev, ldy, sig, sig_scalar, c, cbar, XM, hbuf, wsig ? hbuf + N : nullptr,
+                            G.dX_dev ? E : nullptr, G.dy_dev, G.dsigma2_dev, G.dsigma2 ? dsum : nullptr);
+        if (rc == 0 && G.dsigma2 && ctx->nccl_comm && ctx->nranks > 1) {
+            NcclApi* a = nccl_api();
+            ncclResult_t r = a->AllReduce(dsum, dsum, 1, ncclFloat64, ncclSum, (ncclComm_t)ctx->nccl_comm, ctx->stream);
+            rc = (r != ncclSuccess) ? nccl_fail(ctx, r, "ncclAllReduce") : nccl_async_check(ctx);
+        }
+    }
+    if (rc == 0 && needQ) rc = grad_q(ctx, post, A, ldq, dk);
+    if (rc == 0 && (G.dmw || G.dlambda))
+        rc = grad_prior_multi(ctx, prior, post, diagonal ? lamd : nullptr, A, ldq, U, k, c, cbar, uc, G.dmw ? dmw : nullptr,
+                              G.dlambda ? dlam : nullptr);
+    if (rc == 0 && G.dX_dev) {
+        rc = grad_a_multi(ctx, A, ldq, dk, kp, D, k, M, c, cbar);
+        if (rc == 0) rc = grad_x_multi(ctx, post, x, A, ldq, dk, k, kp, fast, E, sig, sig_scalar, G.dX_dev, G.ld_dX);
+    }
+    if (rc != 0) return done(rc);
     if (G.dmw) e = cudaMemcpyAsync(G.dmw, dmw, (size_t)D * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && G.dlambda)
         e = cudaMemcpyAsync(G.dlambda, dlam, (size_t)ndl * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);

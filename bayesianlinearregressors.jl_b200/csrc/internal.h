@@ -214,8 +214,9 @@ int predict_mean_var(blr_ctx* ctx, blr_post* p, const blr_x* x, const double* si
                      double* mean_dev, double* var_dev);
 int predict_cov(blr_ctx* ctx, blr_post* p, const blr_x* x, const double* sigma2, double sigma2_scalar, double* C_dev);
 int sample_weights(blr_ctx* ctx, blr_post* p, int64_t S, const double* Z_dev, double* W_dev);
+// noiseless: Y = X'Wsamp alone (no draws made, sigma2 / Zy not read)
 int sample_finite(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, int64_t S, const double* sigma2,
-                  double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev);
+                  double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, bool noiseless = false);
 int apply_weights(blr_ctx* ctx, const blr_x* x, const double* w_dev, double* out_dev);
 // C[m, n] = beta * C + Σ_k A[m, k] B[k, n] with arbitrary element strides (small / odd shapes; plain DFMA)
 int gemm_generic(blr_ctx* ctx, int64_t M, int64_t Nn, int64_t K, const double* A, int64_t as_m, int64_t as_k,
@@ -232,7 +233,8 @@ struct RandChunk {
     int64_t ldy, ldz, n_global, N_global;
 };
 int sample_finite_fast(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, int64_t S, const double* sigma2,
-                       double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, const RandChunk* chunk = nullptr);
+                       double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, const RandChunk* chunk = nullptr,
+                       bool noiseless = false);
 int predict_mean_var_fast(blr_ctx* ctx, blr_post* p, const blr_x* x, const double* sigma2, double sigma2_scalar,
                           double* mean_dev, double* var_dev);
 // 2-D tiled TMA map of a column-major fp64 matrix (inner x outer, leading dimension ld), 128-byte swizzled boxes
@@ -254,6 +256,23 @@ int grad_q(blr_ctx* ctx, blr_post* p, double* Qp, int64_t ldq, int64_t dk);
 // dX = -Q X S + m' se'  in x's layout
 int grad_x(blr_ctx* ctx, const blr_post* p, const blr_x* x, const double* Qp, int64_t ldq, int64_t dk, bool fast,
            const double* se, const double* sigma2, double sigma2_scalar, double* dX, int64_t ld_dX);
+// rank k (blr_logpdf_multi_grad), L = Σ_j c_j ℓ_j with c = c_dev (device, k), c̄ = cbar; kp = k rounded up to 16.
+// U (D x k): column 0 is overwritten with m'_0 - mw, columns 1 .. k-1 = W'Z_j (Z = L⁻¹R of the forward pass); M = mw + U
+int grad_means_multi(blr_ctx* ctx, blr_post* p, const double* mw_dev, const double* Z, int64_t k, double* U, double* M);
+// XM (N x k scratch) = X'M; mean, var (N scratch) = x_n'm'_0, h_n (only when dsig / dsig_sum); E (kp x N, point-major; may be
+// null) = residuals; dY (ld ldy), dsig (N) and dsig_sum (device scalar) may be null
+int grad_obs_multi(blr_ctx* ctx, blr_post* p, const blr_x* x, const double* M, int64_t k, int64_t kp, const double* Y, int64_t ldy,
+                   const double* sigma2, double sigma2_scalar, const double* c_dev, double cbar, double* XM, double* mean,
+                   double* var, double* E, double* dY, double* dsig, double* dsig_sum);
+// uc (D scratch) = U c; dmw = Λw U c; dlam = -1/2 (c̄ (Q - Λw⁻¹) + U diag(c) U') or its diagonal; dmw / dlam may be null
+int grad_prior_multi(blr_ctx* ctx, const blr_prior* prior, blr_post* p, const double* lam_dev, const double* Q, int64_t ldq,
+                     const double* U, int64_t k, const double* c_dev, double cbar, double* uc, double* dmw, double* dlam);
+// A (ldq x (dk + kp), Q in its first dk columns) = [-c̄ Q | M diag(c)] in place
+int grad_a_multi(blr_ctx* ctx, double* A, int64_t ldq, int64_t dk, int64_t kp, int64_t D, int64_t k, const double* M,
+                 const double* c_dev, double cbar);
+// dX = S A [X ; E'] in x's layout
+int grad_x_multi(blr_ctx* ctx, const blr_post* p, const blr_x* x, const double* A, int64_t ldq, int64_t dk, int64_t k, int64_t kp,
+                 bool fast, const double* E, const double* sigma2, double sigma2_scalar, double* dX, int64_t ld_dX);
 
 // ---- synth.cu
 int synth_normal(blr_ctx* ctx, double* out, int64_t rows, int64_t cols, int64_t ld, uint64_t seed, uint64_t stream_id,

@@ -502,10 +502,11 @@ __global__ void add_obs_noise_kernel(double* __restrict__ Y, int64_t N, int64_t 
 }
 
 int sample_finite(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, int64_t S, const double* sigma2,
-                  double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev) {
+                  double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, bool noiseless) {
     const int64_t N = x->N, D = x->D;
     if (N == 0 || S == 0) return 0;
-    if (sample_fast_eligible(x)) return sample_finite_fast(ctx, x, Wsamp_dev, S, sigma2, sigma2_scalar, Zy_dev, seed, Y_dev);
+    if (sample_fast_eligible(x))
+        return sample_finite_fast(ctx, x, Wsamp_dev, S, sigma2, sigma2_scalar, Zy_dev, seed, Y_dev, nullptr, noiseless);
     const bool colv = x->layout == BLR_COLVECS;
     if (D >= 64 && N >= 128) {
         // RowVecs, or ColVecs with an odd leading dimension / misaligned base: blocks of points staged into an aligned ColVecs
@@ -534,13 +535,14 @@ int sample_finite(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, int64_t
             const RandChunk ck = {N, N, a, N};
             if (rc == 0)
                 rc = sample_finite_fast(ctx, &sub, Wsamp_dev, S, sigma2 ? sigma2 + a : nullptr, sigma2_scalar,
-                                        Zy_dev ? Zy_dev + a : nullptr, seed, Y_dev + a, &ck);
+                                        Zy_dev ? Zy_dev + a : nullptr, seed, Y_dev + a, &ck, noiseless);
         }
         cudaFreeAsync(stage, ctx->stream);
         return rc;
     }
     // Y (N x S) = X' Wsamp : A[m = n, k = d] = X[d, n]
     BLR_TRY(gemm_generic(ctx, N, S, D, x->p, colv ? x->ld : 1, colv ? 1 : x->ld, Wsamp_dev, 1, D, Y_dev, 1, N, 0.0));
+    if (noiseless) return 0;
     add_obs_noise_kernel<<<(int)std::min<int64_t>((N * S + 255) / 256, (int64_t)ctx->sm_count * 16), 256, 0, ctx->stream>>>(
         Y_dev, N, S, sigma2, sigma2_scalar, Zy_dev, seed);
     BLR_CHECK_LAUNCH(ctx, "add_obs_noise_kernel");

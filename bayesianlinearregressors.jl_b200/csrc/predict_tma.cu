@@ -411,6 +411,7 @@ struct RandParams {
     double sigma2_scalar;
     const double* Zy;   // N x S column-major, or null
     uint64_t seed;
+    bool noise;         // false: Y = X'W alone (no draws, sigma2 / Zy not read)
     double* Y;          // N x S column-major
     int64_t ldy, ldz;   // leading dimensions of Y and Zy (two-group kernel; the single-group kernel uses N for both)
     int64_t n_global;   // index of this launch's first point in the whole problem and the whole problem's N: the Philox counter
@@ -509,18 +510,20 @@ __global__ void __launch_bounds__(rk::THREADS, 1) rand_tma_kernel(const RandPara
             for (int mi = 0; mi < 4; ++mi) {
                 const int64_t n = p0 + wm * 32 + mi * 8 + g;
                 if (n < p.N) {
-                    const double sd = sqrt(p.sigma2 ? p.sigma2[n] : p.sigma2_scalar);
+                    const double sd = p.noise ? sqrt(p.sigma2 ? p.sigma2[n] : p.sigma2_scalar) : 0.0;
 #pragma unroll
                     for (int ni = 0; ni < 4; ++ni) {
                         const int s0 = sb * TS + wn * 32 + ni * 8 + kq * 2;  // even
                         if (s0 < p.S) {
-                            double z0, z1;
-                            if (p.Zy) {
-                                z0 = p.Zy[(int64_t)s0 * p.ldz + n];
-                                z1 = (s0 + 1 < p.S) ? p.Zy[(int64_t)(s0 + 1) * p.ldz + n] : 0.0;
-                            } else {
-                                philox_normal_pair(p.seed, 7, (uint64_t)(p.n_global + n) + (uint64_t)(s0 >> 1) * (uint64_t)p.N_global, z0,
-                                                   z1);
+                            double z0 = 0.0, z1 = 0.0;
+                            if (p.noise) {
+                                if (p.Zy) {
+                                    z0 = p.Zy[(int64_t)s0 * p.ldz + n];
+                                    z1 = (s0 + 1 < p.S) ? p.Zy[(int64_t)(s0 + 1) * p.ldz + n] : 0.0;
+                                } else {
+                                    philox_normal_pair(p.seed, 7, (uint64_t)(p.n_global + n) + (uint64_t)(s0 >> 1) * (uint64_t)p.N_global,
+                                                       z0, z1);
+                                }
                             }
                             p.Y[(int64_t)s0 * p.ldy + n] = fma(sd, z0, acc[mi][ni][0]);
                             if (s0 + 1 < p.S) p.Y[(int64_t)(s0 + 1) * p.ldy + n] = fma(sd, z1, acc[mi][ni][1]);
@@ -557,10 +560,11 @@ bool sample_fast_eligible(const blr_x* x) {
 // chunk != nullptr: x holds points [n_global, n_global + x->N) of a problem of N_global points (a staged block of an input the
 // tensor map cannot address); sigma2 / Zy_dev / Y_dev already point at the block's first point, ldy / ldz span the whole problem.
 int sample_finite_fast(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, int64_t S, const double* sigma2,
-                       double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, const RandChunk* chunk) {
+                       double sigma2_scalar, const double* Zy_dev, uint64_t seed, double* Y_dev, const RandChunk* chunk,
+                       bool noiseless) {
     const int D = (int)x->D;
     // the two-group kernel reads the sample weights through a tensor map over the D x S matrix itself: D must be even
-    if (!chunk && (D % 2) == 0 && (ctx->rand_pp == 2 || (ctx->rand_pp == 1 && Zy_dev != nullptr))) {
+    if (!noiseless && !chunk && (D % 2) == 0 && (ctx->rand_pp == 2 || (ctx->rand_pp == 1 && Zy_dev != nullptr))) {
         const int r = sample_finite_pp(ctx, x, Wsamp_dev, S, sigma2, sigma2_scalar, Zy_dev, seed, Y_dev);
         if (r <= 0) return r;  // 1: weights not 16-byte aligned -> the default kernel
     }
@@ -580,6 +584,7 @@ int sample_finite_fast(blr_ctx* ctx, const blr_x* x, const double* Wsamp_dev, in
     rp.sigma2_scalar = sigma2_scalar;
     rp.Zy = Zy_dev;
     rp.seed = seed;
+    rp.noise = !noiseless;
     rp.Y = Y_dev;
     rp.ldy = chunk ? chunk->ldy : x->N;
     rp.ldz = chunk ? chunk->ldz : x->N;
@@ -793,6 +798,7 @@ static int launch_rand_pp(blr_ctx* ctx, const blr_x* x, int64_t n0, int64_t cnt,
     rp_.sigma2_scalar = sigma2_scalar;
     rp_.Zy = Zy;
     rp_.seed = seed;
+    rp_.noise = true;
     rp_.Y = Y_dev + n0;
     rp_.ldy = x->N;
     rp_.ldz = ldz;

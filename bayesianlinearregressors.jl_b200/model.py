@@ -374,10 +374,13 @@ def _logpdf_multi(fx: FiniteGP, Y) -> np.ndarray:
 GRAD_KEYS = ("X", "y", "σ²", "mw", "Λw")
 
 
-def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatrix, yv: DeviceVector, Σy, wrt, out_like=None):
-    """One blr_logpdf_grad call.  Per-observation gradients are written into CUDA tensors on out_like's device when
-    `out_like` (a CUDA tensor) is given -- dX with the shape torch sees x in, (N, D) for ColVecs -- else downloaded into numpy
-    arrays (dX with the Julia-side shape).  Keys of `wrt` not in GRAD_KEYS are an error; keys left out get NULL."""
+def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatrix, yv, Σy, wrt, out_like=None, k=None,
+                      weights=None):
+    """One blr_logpdf_grad call, or with `k` one blr_logpdf_multi_grad call: then yv is the device address of Y (N x k,
+    column-major, ld = N), the value is the k log densities and the gradients are those of Σ_j weights_j ℓ_j (weights: None for
+    all ones).  Per-observation gradients are written into CUDA tensors on out_like's device when `out_like` (a CUDA tensor) is
+    given -- dX with the shape torch sees x in, (N, D) for ColVecs; "y" (N, k) -- else downloaded into numpy arrays (dX with the
+    Julia-side shape).  Keys of `wrt` not in GRAD_KEYS are an error; keys left out get NULL."""
     wrt = tuple(wrt)
     bad = [k for k in wrt if k not in GRAD_KEYS]
     if bad:
@@ -385,7 +388,7 @@ def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatri
     D = blr.mw.shape[0]
     if X.D != D:  # `X' * mw` (:33) throws DimensionMismatch in the reference
         raise L.DimensionMismatch(L.E_DIM, "size(X, 1) != length(mw)")
-    if yv.n != X.N:  # src/bayesian_linear_regression.jl:74
+    if k is None and yv.n != X.N:  # src/bayesian_linear_regression.jl:74
         raise L.DimensionMismatch(L.E_DIM, "length(y) != size(fx.x.X, 2)")
     noise, keep_noise = make_noise(ctx, Σy, X.N)
     prior, keep_prior = blr._prior_struct()
@@ -415,7 +418,7 @@ def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatri
         return b.data_ptr() if out_like is not None else b.device_ptr()
 
     if "y" in wrt:
-        dev["y"] = buf(N)
+        dev["y"] = buf(N) if k is None else buf(k, N)  # (k, N) row-major == N x k column-major
         g.dy_dev = addr(dev["y"])
     if "σ²" in wrt and vector_noise:
         dev["σ²"] = buf(N)
@@ -426,36 +429,74 @@ def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatri
         g.ld_dX = max(D if colv else N, 1)
     if out_like is not None:  # the output tensors were just allocated on torch's stream
         ctx.wait_torch_stream(out_like)
-    lp = C.c_double()
-    ctx.check(ctx.lib.blr_logpdf_grad(ctx.handle, C.byref(prior), X.handle, yv.handle, C.byref(noise), C.byref(lp), C.byref(g)))
+    if k is None:
+        lp = C.c_double()
+        ctx.check(ctx.lib.blr_logpdf_grad(ctx.handle, C.byref(prior), X.handle, yv.handle, C.byref(noise), C.byref(lp), C.byref(g)))
+        lp = lp.value
+    else:
+        lp = np.empty(k)
+        c = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64).reshape(k)
+        ctx.check(ctx.lib.blr_logpdf_multi_grad(ctx.handle, C.byref(prior), X.handle, yv, max(N, 1), k, C.byref(noise),
+                                                None if c is None else c.ctypes.data_as(L.c_double_p), lp.ctypes.data_as(L.c_double_p),
+                                                C.byref(g)))
     if "σ²" in wrt and not vector_noise:
         out["σ²"] = dσ2_host.value
     if out_like is not None:
         ctx.release_to_torch_stream(out_like.device)
+        if k is not None and "y" in dev:
+            dev["y"] = dev["y"].T
         out.update(dev)
     else:
-        for k, v in dev.items():
+        for key, v in dev.items():
             a = v.download()
-            out[k] = a.reshape((D, N) if colv else (N, D), order="F") if k == "X" else a
-    return lp.value, out
+            if key == "X":
+                a = a.reshape((D, N) if colv else (N, D), order="F")
+            elif key == "y" and k is not None:
+                a = a.reshape((N, k), order="F")
+            out[key] = a
+    return lp, out
 
 
-def logpdf_and_grad(fx: FiniteGP, y, wrt=GRAD_KEYS):
+def logpdf_and_grad(fx: FiniteGP, y, wrt=GRAD_KEYS, weights=None):
     """logpdf(fx, y) and its gradients with respect to the keys of `wrt` -- "X" (the inputs; ϕ(x) for a BasisFunctionRegressor),
     "y", "σ²" (a scalar for scalar noise, else one per observation), "mw" and "Λw" (D values for a Diagonal prior, else the
     symmetric D x D G with dℓ = <G, dΛw>) -- in closed form on the device (blr_logpdf_grad).  Returns (logpdf, dict).
     Per-observation gradients of inputs given as CUDA tensors come back as CUDA tensors (dX with x's tensor shape, (N, D) for
-    ColVecs); otherwise everything is numpy (dX D x N for ColVecs, N x D for RowVecs)."""
+    ColVecs); otherwise everything is numpy (dX D x N for ColVecs, N x D for RowVecs).
+    A matrix `Y` (N x k, a host array or a CUDA tensor; one observation vector per column) returns the k log densities and the
+    gradients of Σ_j weights_j ℓ_j (weights: k values, None for all ones) from ONE call (blr_logpdf_multi_grad): the Gram pass and
+    the O(N D²) product run once for all k columns.  "y" then has Y's shape."""
     fx = _to_finite_blr(fx)
     ctx = fx._context()
-    X = x_as_colvecs(ctx, fx.x)
-    yv = _as_device_vector(ctx, y)
     out_like = None
     for cand in (fx.x.X, y):
         if _is_torch_cuda(cand):
             out_like = cand
             break
+    if (isinstance(y, np.ndarray) or _is_torch_cuda(y)) and y.ndim == 2:
+        return _logpdf_multi_grad(ctx, fx, y, wrt, weights, out_like)
+    X = x_as_colvecs(ctx, fx.x)
+    yv = _as_device_vector(ctx, y)
     return _logpdf_grad_call(ctx, fx.f, X, yv, fx.Σy, wrt, out_like)
+
+
+def _logpdf_multi_grad(ctx: Context, fx: FiniteGP, Y, wrt, weights, out_like):
+    X = x_as_colvecs(ctx, fx.x)
+    k = int(Y.shape[1])
+    if X.D != fx.f.mw.shape[0]:
+        raise L.DimensionMismatch(L.E_DIM, "size(X, 1) != length(mw)")
+    if Y.shape[0] != X.N:  # src/bayesian_linear_regression.jl:74
+        raise L.DimensionMismatch(L.E_DIM, "length(y) != size(fx.x.X, 2)")
+    if weights is not None and np.size(weights) != k:
+        raise L.DimensionMismatch(L.E_DIM, "length(weights) != size(Y, 2)")
+    if _is_torch_cuda(Y):
+        import torch
+
+        Yt = Y.to(torch.float64).T.contiguous()  # (k, N) row-major == N x k column-major
+        ctx.wait_torch_stream()
+        return _logpdf_grad_call(ctx, fx.f, X, C.c_void_p(Yt.data_ptr()), fx.Σy, wrt, out_like, k, weights)
+    Yd = DeviceVector.upload(ctx, np.asarray(Y, dtype=np.float64).T.reshape(-1))  # column-major N x k, flattened
+    return _logpdf_grad_call(ctx, fx.f, X, C.c_void_p(Yd.device_ptr()), fx.Σy, wrt, out_like, k, weights)
 
 
 def _torch_logpdf_function():
@@ -495,7 +536,50 @@ def _torch_logpdf_function():
             saved = fctx.saved_tensors
             return tuple(grad_out * v if present else None for v, present in zip(saved, fctx.present))
 
-    return TorchLogpdf
+    class TorchLogpdfMulti(torch.autograd.Function):
+        """The k log densities of the columns of an (N, k) Y as a differentiable torch op.  The cotangent is not known in the
+        forward call, so forward runs blr_logpdf_multi alone and backward makes one blr_logpdf_multi_grad call with the
+        cotangent as the weights: the backward re-runs the Gram pass and the factorisation."""
+
+        @staticmethod
+        def forward(fctx, X, Y, mw, Λw, σ2):
+            if not (X.is_cuda and X.dtype == torch.float64 and X.dim() == 2):
+                raise L.BLRError(L.E_INVALID, "torch_logpdf: X must be an (N, D) float64 CUDA tensor")
+            fx = _torch_finite_gp(X, mw, Λw, σ2)
+            fctx.save_for_backward(X, Y, mw, Λw, σ2)
+            return torch.as_tensor(_logpdf_multi(fx, Y.detach()), dtype=torch.float64, device=X.device)
+
+        @staticmethod
+        def backward(fctx, grad_out):
+            X, Y, mw, Λw, σ2 = fctx.saved_tensors
+            need = fctx.needs_input_grad
+            wrt = [k for k, n in zip(GRAD_KEYS, (need[0], need[1], need[4], need[2], need[3])) if n]
+            if not wrt:
+                return (None,) * 5
+            fx = _torch_finite_gp(X, mw, Λw, σ2)
+            c = grad_out.detach().to("cpu", torch.float64).numpy()
+            _, g = logpdf_and_grad(fx, Y.detach(), wrt=wrt, weights=c)
+            grads = []
+            for k, like in (("X", X), ("y", Y), ("mw", mw), ("Λw", Λw), ("σ²", σ2)):
+                v = g.get(k)
+                if v is not None and not isinstance(v, torch.Tensor):
+                    v = torch.as_tensor(np.asarray(v), dtype=torch.float64, device=like.device).reshape(like.shape)
+                grads.append(v)
+            return tuple(grads)
+
+    return TorchLogpdf, TorchLogpdfMulti
+
+
+def _torch_finite_gp(X, mw, Λw, σ2):
+    """BayesianLinearRegressor(mw, Λw)(ColVecs(X), σ²) over detached tensors: the prior on the host, X and a vector σ² on the
+    device."""
+    import torch
+
+    mw_h = mw.detach().to("cpu", torch.float64).numpy()
+    lam_h = Λw.detach().to("cpu", torch.float64).numpy()
+    blr = BayesianLinearRegressor(mw_h, Diagonal(lam_h) if lam_h.ndim == 1 else lam_h)
+    Σy = float(σ2) if σ2.dim() == 0 else σ2.detach().to(torch.float64).contiguous()
+    return blr(ColVecs(X.detach().contiguous()), Σy)
 
 
 _TORCH_LOGPDF = None
@@ -505,11 +589,14 @@ def torch_logpdf(X, y, mw, Λw, σ2):
     """Differentiable logpdf of y under BayesianLinearRegressor(mw, Λw)(ColVecs(X), σ²) for float64 CUDA tensors: X is (N, D),
     Λw is (D,) (Diagonal prior) or (D, D), σ² is 0-d (scalar noise) or (N,).  The gradients of the inputs that require them are
     computed on the device in the forward call; this is what makes a TorchFeatureMap's network trainable by type-II maximum
-    likelihood (the reference's examples/nn-blr.jl)."""
+    likelihood (the reference's examples/nn-blr.jl).
+    An (N, k) y (k target series sharing one feature map) returns the (k,) log densities.  Its forward is blr_logpdf_multi; its
+    backward is one blr_logpdf_multi_grad call weighted by the incoming gradient, which re-runs the Gram pass (about the cost of
+    one single-column gradient call, whatever k)."""
     global _TORCH_LOGPDF
     if _TORCH_LOGPDF is None:
         _TORCH_LOGPDF = _torch_logpdf_function()
-    return _TORCH_LOGPDF.apply(X, y, mw, Λw, σ2)
+    return _TORCH_LOGPDF[1 if y.dim() == 2 else 0].apply(X, y, mw, Λw, σ2)
 
 
 def posterior(fx: FiniteGP, y):

@@ -223,6 +223,19 @@ typedef struct blr_logpdf_grads {
 } blr_logpdf_grads;
 int blr_logpdf_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const blr_vec* y, const blr_noise* noise,
                     double* logpdf_out, const blr_logpdf_grads* g);
+/* Gradients of L = Σ_j c_j ℓ_j, ℓ_j the log marginal likelihood of column j of Y (blr_logpdf_multi), c = weights (host, k;
+ * NULL = all ones: a reverse-mode rule passes its cotangent here).  With c̄ = Σ_j c_j, m'_j the posterior mean of column j,
+ * M' = [m'_1 .. m'_k], u_j = m'_j - mw, U = [u_1 .. u_k] and e_jn = y_jn - x_n'm'_j (each line the single-column formula summed):
+ *   ∂/∂x_n = s_n (Σ_j c_j e_jn m'_j - c̄ Q x_n)    ∂/∂Y[n, j] = -c_j s_n e_jn
+ *   ∂/∂σ²_n = (s_n² (c̄ x_n'Q x_n + Σ_j c_j e_jn²) - c̄ s_n) / 2
+ *   ∂/∂mw  = Λw U c                                ∂/∂Λw = -(c̄ (Q - Λw⁻¹) + U diag(c) U') / 2  (its diagonal for a Diagonal prior)
+ * g is a blr_logpdf_grads whose dy_dev is N x k column-major with leading dimension ldy, like Y_dev; every other field as for
+ * blr_logpdf_grad.  logpdf_out (host, k; may be NULL) is bit-identical to blr_logpdf_multi's.  k == 0 writes zeros to every
+ * requested output.  The O(N D²) work is one GEMM over [X ; E'] with K = D + k rounded up to 16, so k columns cost about one
+ * blr_logpdf_grad call, not k.  Scalar / vector Σy only; per-observation outputs cover this rank's shard, the others are
+ * replicated on every rank. */
+int blr_logpdf_multi_grad(blr_ctx* ctx, const blr_prior* prior, const blr_x* x, const double* Y_dev, int64_t ldy, int64_t k,
+                          const blr_noise* noise, const double* weights, double* logpdf_out, const blr_logpdf_grads* g);
 
 /* ------------------------------------------------------------------ prediction / sampling
  * replaces mean / var / mean_and_var / rand, src/bayesian_linear_regression.jl:33-53,

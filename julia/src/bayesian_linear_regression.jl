@@ -103,6 +103,32 @@ function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteBLR, y::Ab
     return lp, logpdf_pullback
 end
 
+# The same rule for the matrix method above (k observation vectors, one per column of Y): the primal is that method
+# (blr_logpdf_multi); the cotangent Δ of the k values is not known until the pullback, which makes ONE blr_logpdf_multi_grad
+# call with the weights Δ (re-running the Gram pass) -- the gradients of Σ_j Δ_j logpdf_j, in the tangent structure of the
+# vector rule.  Dense Σy: the pullback raises the library's error.
+function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteBLR, Y::AbstractMatrix{<:Real})
+    lps = AbstractGPs.logpdf(fx, Y)
+    function logpdf_multi_pullback(Δ)
+        Δ = collect(Float64, ChainRulesCore.unthunk(Δ))
+        ctx = LibBLR.default_context()
+        prior, keep1 = _prior(fx.f)
+        x = _device_x(ctx, fx.x)
+        noise, keep2 = _noise(ctx, fx.Σy)
+        layout = fx.x isa ColVecs ? LibBLR.COLVECS : LibBLR.ROWVECS
+        dX, dY, dσ², dmw, dΛ = GC.@preserve keep1 keep2 x LibBLR.logpdf_multi_grad(ctx, prior, x, layout, Matrix{Float64}(Y), noise,
+                                                                                      Δ; diagonal=fx.f.Λw isa Diagonal)
+        Λ̄ = fx.f.Λw isa Diagonal ? ChainRulesCore.Tangent{typeof(fx.f.Λw)}(diag=dΛ) : dΛ
+        Σ̄ = fx.Σy isa Diagonal{<:Real,<:FillArrays.Fill} ?
+            ChainRulesCore.Tangent{typeof(fx.Σy)}(diag=ChainRulesCore.Tangent{typeof(fx.Σy.diag)}(value=dσ²)) :
+            ChainRulesCore.Tangent{typeof(fx.Σy)}(diag=dσ²)
+        f̄ = ChainRulesCore.Tangent{typeof(fx.f)}(mw=dmw, Λw=Λ̄)
+        x̄ = ChainRulesCore.Tangent{typeof(fx.x)}(X=dX)
+        return ChainRulesCore.NoTangent(), ChainRulesCore.Tangent{typeof(fx)}(f=f̄, x=x̄, Σy=Σ̄), dY
+    end
+    return lps, logpdf_multi_pullback
+end
+
 function AbstractGPs.posterior(fx::FiniteBLR, y::AbstractVector{<:Real})                           # :60-69
     _, m′, Λ′, T, p = _infer(fx, y; want_T=fx.f.Λw isa AbstractPDMat)
     _POST_CACHE[Λ′] = (copy(m′), p)          # the returned regressor carries its device factor (keyed by its Λ′ array)

@@ -185,6 +185,35 @@ function logpdf_grad(ctx::Context, prior::Prior, x::DeviceX, layout::Cint, y::De
     return lp[], dX, _download(ctx, hy, N), dσ², dmw, dΛ
 end
 
+# gradients of Σ_j Δ_j logpdf(fx, Y[:, j]) (blr_logpdf_multi_grad): one call for all k columns; Δ is the cotangent of the k
+# log densities.  Returns (dX (shaped like the input matrix), dY (N x k), dσ², dmw, dΛw), as logpdf_grad without the value.
+function logpdf_multi_grad(ctx::Context, prior::Prior, x::DeviceX, layout::Cint, Y::Matrix{Float64}, noise::Noise,
+                           Δ::Vector{Float64}; diagonal::Bool)
+    D, N = x.D, x.N
+    k = size(Y, 2)
+    length(Δ) == k || throw(DimensionMismatch("length(Δ) != size(Y, 2)"))
+    Yd = upload_vec(ctx, vec(Y))                       # column-major N x k, ld = N
+    pY = Ref{Ptr{Float64}}(C_NULL)
+    check(ctx, ccall((:blr_vec_device_ptr, libblr), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ref{Ptr{Float64}}), ctx.ptr, Yd.ptr, pY))
+    dmw = Vector{Float64}(undef, D)
+    dΛ = diagonal ? Vector{Float64}(undef, D) : Matrix{Float64}(undef, D, D)
+    dσ²_host = Ref{Float64}(NaN)
+    vector_noise = noise.kind == NOISE_VECTOR
+    hX, pX = _alloc_vec(ctx, D * N)
+    hy, py = _alloc_vec(ctx, N * k)
+    hs, ps = vector_noise ? _alloc_vec(ctx, N) : (nothing, Ptr{Float64}(C_NULL))
+    GC.@preserve Yd Δ dmw dΛ dσ²_host begin
+        g = LogpdfGrads(pointer(dmw), pointer(dΛ), vector_noise ? C_NULL : Base.unsafe_convert(Ptr{Float64}, dσ²_host), ps, py, pX,
+                        max(layout == COLVECS ? D : N, 1))
+        check(ctx, ccall((:blr_logpdf_multi_grad, libblr), Cint,
+            (Ptr{Cvoid}, Ref{Prior}, Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Ref{Noise}, Ptr{Float64}, Ptr{Float64}, Ref{LogpdfGrads}),
+            ctx.ptr, prior, x.ptr, pY[], max(N, 1), k, noise, Δ, C_NULL, g))
+    end
+    dX = reshape(_download(ctx, hX, D * N), layout == COLVECS ? (D, N) : (N, D))
+    dσ² = vector_noise ? _download(ctx, hs, N) : dσ²_host[]
+    return dX, reshape(_download(ctx, hy, N * k), N, k), dσ², dmw, dΛ
+end
+
 # the same from host arrays: blr_stats_create -> blr_stats_accumulate_host -> blr_stats_allreduce -> blr_infer_from_stats
 function infer_host(ctx::Context, prior::Prior, X::StridedMatrix{Float64}, layout::Cint, y::Vector{Float64}, Σy;
                     want_T::Bool=false, chunk::Integer=1 << 16)

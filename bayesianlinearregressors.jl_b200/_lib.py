@@ -76,6 +76,8 @@ SIGNATURES = {
     "blr_vec_synth_targets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int64, C.c_void_p]),
     "blr_x_rff": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, c_void_pp]),
     "blr_x_features": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_double, c_void_pp]),
+    "blr_x_features_vjp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_void_p,
+                                     C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
     "blr_stats_create": (C.c_int, [C.c_void_p, C.c_int64, c_void_pp]),
     "blr_stats_free": (C.c_int, [C.c_void_p, C.c_void_p]),
     "blr_stats_zero": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -679,6 +679,54 @@ int blr_x_rff(blr_ctx* ctx, const blr_x* xin, const double* W, const double* b, 
     return blr_x_features(ctx, xin, W, b, D, BLR_ACT_COS, sqrt(2.0 / (double)(D > 0 ? D : 1)), out);
 }
 
+int blr_x_features_vjp(blr_ctx* ctx, const blr_x* xin, const double* W, const double* b, int64_t D, int act, double scale,
+                       const double* dphi_dev, int64_t ld_dphi, double* dW_host, double* db_host, double* dxin_dev, int64_t ld_dxin) {
+    CTX_ENTER(ctx);
+    if (!xin || !W || !b || !dphi_dev || D < 1) return set_err(ctx, BLR_E_INVALID, "bad feature-map VJP arguments");
+    if (xin->layout != BLR_COLVECS) return set_err(ctx, BLR_E_INVALID, "device feature maps expect ColVecs inputs");
+    const int64_t din = xin->D, N = xin->N;
+    if (din < 1 || din > 384) return set_err(ctx, BLR_E_INVALID, "device feature map: d_in must be 1 .. 384");
+    if (act < BLR_ACT_COS || act > BLR_ACT_SIN) return set_err(ctx, BLR_E_INVALID, "unknown activation");
+    if (ld_dphi < D) return set_err(ctx, BLR_E_INVALID, "ld_dphi too small");
+    if (dxin_dev && ld_dxin < din) return set_err(ctx, BLR_E_INVALID, "ld_dxin too small");
+    const bool want_wb = dW_host || db_host;
+    if (!want_wb && !dxin_dev) return 0;
+
+    // device scratch: [W (D x d_in) | b (D) | dW, db (D x (d_in + 1)) | per-range partials (S x D x (d_in + 1))]
+    const int64_t len = D * (din + 1);
+    const int S = (want_wb && N > 0) ? features_vjp_splits(ctx, N, D, din) : 0;
+    double* buf = nullptr;
+    BLR_CUDA_OK(ctx, dev_alloc(ctx, &buf, (size_t)(D * din + D + (want_wb ? len * (1 + S) : 0)) * sizeof(double)));
+    double *Wd = buf, *bd = Wd + D * din, *dWb = bd + D, *ws = dWb + len;
+    auto done = [&](int rc) {
+        dev_free(ctx->stream, buf);
+        return rc;
+    };
+    cudaError_t e = cudaMemcpyAsync(Wd, W, (size_t)D * din * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(bd, b, (size_t)D * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && want_wb && N == 0) e = cudaMemsetAsync(dWb, 0, (size_t)len * sizeof(double), ctx->stream);
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "feature-map VJP upload"));
+    if (N > 0) {
+        const int rc = features_vjp(ctx, xin, Wd, bd, D, act, scale, dphi_dev, ld_dphi, want_wb ? dWb : nullptr, ws, S, dW_host != nullptr,
+                                    dxin_dev, ld_dxin);
+        if (rc != 0) return done(rc);
+    }
+    if (want_wb && ctx->nccl_comm && ctx->nranks > 1) {
+        // [dW | db] in one all-reduce, or the db column alone when dW is not requested
+        const int64_t off = dW_host ? 0 : D * din;
+        NcclApi* a = nccl_api();
+        ncclResult_t r = a->AllReduce(dWb + off, dWb + off, (size_t)(len - off), ncclFloat64, ncclSum, (ncclComm_t)ctx->nccl_comm,
+                                      ctx->stream);
+        const int rc = (r != ncclSuccess) ? nccl_fail(ctx, r, "ncclAllReduce") : nccl_async_check(ctx);
+        if (rc != 0) return done(rc);
+    }
+    if (dW_host) e = cudaMemcpyAsync(dW_host, dWb, (size_t)D * din * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && db_host) e = cudaMemcpyAsync(db_host, dWb + D * din, (size_t)D * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return done(cuda_fail(ctx, e, "download feature-map gradients"));
+    return done(0);
+}
+
 // ---------------------------------------------------------------------------------------------- inference
 int blr_stats_create(blr_ctx* ctx, int64_t D, blr_stats** out) {
     CTX_ENTER(ctx);

@@ -285,6 +285,14 @@ int rff_features(blr_ctx* ctx, const blr_x* xin, const double* W_dev, const doub
                  int64_t ldo);
 int transpose_to_colvecs(blr_ctx* ctx, const blr_x* x, double* out, int64_t ldo);
 
+// ---- features_grad.cu: VJP of affine_features for the cotangent dphi (D x N, leading dimension ldp).  dWb (may be null) =
+// [dW (D x d_in) | db (D)], column-major, from S point ranges through ws (S x D x (d_in + 1)); with_w = false computes and writes
+// only the db part.
+// dx (may be null) = W'g, d_in x N with leading dimension lddx.  S from features_vjp_splits.
+int features_vjp_splits(const blr_ctx* ctx, int64_t N, int64_t D, int64_t din);
+int features_vjp(blr_ctx* ctx, const blr_x* xin, const double* W_dev, const double* b_dev, int64_t D, int act, double scale,
+                 const double* dphi, int64_t ldp, double* dWb, double* ws, int S, bool with_w, double* dx, int64_t lddx);
+
 // ---- calib.cu
 int calib_dmma(blr_ctx* ctx, double* tflops);
 int calib_dfma(blr_ctx* ctx, double* tflops);

@@ -198,7 +198,47 @@ def _to_finite_blr(fx: FiniteGP) -> FiniteGP:
     return fx
 
 
-class RandomFourierFeatures:
+FEATURE_GRAD_KEYS = ("W", "b", "xin")
+
+
+class _DeviceAffineMap:
+    """What the two device-native maps ϕ(x) = scale * act(W x + b) share: input staging and the vector-Jacobian product."""
+
+    ACTS = {"cos": 0, "tanh": 1, "relu": 2, "identity": 3, "sin": 4}
+
+    def _context(self) -> Context:
+        return self.ctx if self.ctx is not None else default_context()
+
+    def _device_inputs(self, ctx: Context, x) -> DeviceMatrix:
+        x = _wrap_inputs(x)
+        if isinstance(x, RowVecs):
+            x = ColVecs(np.ascontiguousarray(np.asarray(x.X).T)) if isinstance(x.X, np.ndarray) else x
+        return x_as_colvecs(ctx, x)
+
+    def vjp(self, x, dΦ, wrt=FEATURE_GRAD_KEYS):
+        """Vector-Jacobian product of ϕ at x for the cotangent dΦ (blr_x_features_vjp): with z = W x + b and
+        g = dΦ * scale * act'(z), "W" = g x' (D x d_in numpy), "b" = Σ_n g_n (length D), "xin" = W'g (d_in x N numpy for host
+        x, an (N, d_in) CUDA tensor for a torch x).  dΦ is D x N numpy or an (N, D) CUDA tensor (ϕ(x)'s ColVecs convention)."""
+        ctx = self._context()
+        xin = self._device_inputs(ctx, x)
+        if _is_torch_cuda(dΦ):
+            import torch
+
+            if not (dΦ.dim() == 2 and dΦ.stride(1) == 1):
+                dΦ = dΦ.contiguous()
+            d = dΦ.to(torch.float64)
+            if tuple(d.shape) != (xin.N, self.W.shape[0]):
+                raise L.DimensionMismatch(L.E_DIM, "dΦ must be an (N, D) tensor")
+            ctx.wait_torch_stream(d)
+            return _features_vjp(ctx, self, xin, d.data_ptr(), max(d.stride(0), 1), wrt, _torch_of(x))
+        Φd = DeviceMatrix.upload(ctx, np.asarray(dΦ, dtype=np.float64), L.COLVECS)
+        if Φd.D != self.W.shape[0] or Φd.N != xin.N:
+            raise L.DimensionMismatch(L.E_DIM, "size(dΦ) != (D, N)")
+        ptr, ld = Φd.device_ptr()
+        return _features_vjp(ctx, self, xin, ptr, ld, wrt, _torch_of(x))
+
+
+class RandomFourierFeatures(_DeviceAffineMap):
     """Device-native feature map ϕ(x) = sqrt(2/D) cos(W x + b) for BasisFunctionRegressor (BASELINE config 5).
     W is D x d_in, b has length D; input ColVecs (d_in x N) -> output ColVecs (D x N) resident on the device."""
 
@@ -206,24 +246,20 @@ class RandomFourierFeatures:
         self.W = _f64(np.asarray(W, dtype=np.float64), "F")
         self.b = _f64(np.asarray(b, dtype=np.float64).reshape(-1))
         self.ctx = ctx
+        self.act, self.scale = "cos", float(np.sqrt(2.0 / max(self.W.shape[0], 1)))
 
     def __call__(self, x):
-        ctx = self.ctx if self.ctx is not None else default_context()
-        x = _wrap_inputs(x)
-        if isinstance(x, RowVecs):
-            x = ColVecs(np.ascontiguousarray(np.asarray(x.X).T)) if isinstance(x.X, np.ndarray) else x
-        xin = x_as_colvecs(ctx, x)
+        ctx = self._context()
+        xin = self._device_inputs(ctx, x)
         h = C.c_void_p()
         ctx.check(ctx.lib.blr_x_rff(ctx.handle, xin.handle, _ptr(self.W), _ptr(self.b), self.W.shape[0], C.byref(h)))
         return ColVecs(DeviceMatrix(ctx, h, self.W.shape[0], xin.N, L.COLVECS))
 
 
-class AffineFeatures:
+class AffineFeatures(_DeviceAffineMap):
     """Device-native one-layer feature map ϕ(x) = scale * act(W x + b) (blr_x_features): random Fourier features are
     act = "cos", scale = sqrt(2/D); "tanh" / "relu" give the last-layer features of examples/nn-blr.jl style models;
     "identity" a linear projection.  Output resident on the device like RandomFourierFeatures."""
-
-    ACTS = {"cos": 0, "tanh": 1, "relu": 2, "identity": 3, "sin": 4}
 
     def __init__(self, W, b, act: str = "tanh", scale: float = 1.0, ctx: Optional[Context] = None):
         if act not in self.ACTS:
@@ -233,17 +269,60 @@ class AffineFeatures:
         self.act, self.scale, self.ctx = act, float(scale), ctx
 
     def __call__(self, x):
-        ctx = self.ctx if self.ctx is not None else default_context()
-        x = _wrap_inputs(x)
-        if isinstance(x, RowVecs):
-            x = ColVecs(np.ascontiguousarray(np.asarray(x.X).T)) if isinstance(x.X, np.ndarray) else x
-        xin = x_as_colvecs(ctx, x)
+        ctx = self._context()
+        xin = self._device_inputs(ctx, x)
         if xin.D != self.W.shape[1]:
             raise L.DimensionMismatch(L.E_DIM, "size(W, 2) != size(x, 1)")
         h = C.c_void_p()
         ctx.check(ctx.lib.blr_x_features(ctx.handle, xin.handle, _ptr(self.W), _ptr(self.b), self.W.shape[0], self.ACTS[self.act],
                                          self.scale, C.byref(h)))
         return ColVecs(DeviceMatrix(ctx, h, self.W.shape[0], xin.N, L.COLVECS))
+
+
+def _torch_of(x):
+    """The CUDA tensor behind inputs x, or None."""
+    x = _wrap_inputs(x)
+    X = x.X if isinstance(x, (ColVecs, RowVecs)) else x
+    return X if _is_torch_cuda(X) else None
+
+
+def _features_vjp(ctx: Context, ϕ: _DeviceAffineMap, xin: DeviceMatrix, dphi_ptr: int, ld_dphi: int, wrt, x_torch=None):
+    """One blr_x_features_vjp call for the cotangent at device address dphi_ptr (D x N, leading dimension ld_dphi)."""
+    wrt = tuple(wrt)
+    bad = [k for k in wrt if k not in FEATURE_GRAD_KEYS]
+    if bad:
+        raise L.BLRError(L.E_INVALID, f"unknown feature-map gradient keys {bad}; expected a subset of {FEATURE_GRAD_KEYS}")
+    D, din, N = ϕ.W.shape[0], ϕ.W.shape[1], xin.N
+    if xin.D != din:
+        raise L.DimensionMismatch(L.E_DIM, "size(W, 2) != size(x, 1)")
+    out = {}
+    if "W" in wrt:
+        out["W"] = np.empty((D, din), order="F")
+    if "b" in wrt:
+        out["b"] = np.empty(D)
+    dx, dx_ptr = None, None
+    if "xin" in wrt and N > 0:
+        if x_torch is not None:
+            import torch
+
+            dx = torch.empty((N, din), dtype=torch.float64, device=x_torch.device)  # (N, d_in) row-major == d_in x N ColVecs
+            ctx.wait_torch_stream(dx)
+            dx_ptr = dx.data_ptr()
+        else:
+            dx = DeviceVector.alloc(ctx, N * din)
+            dx_ptr = dx.device_ptr()
+    ctx.check(ctx.lib.blr_x_features_vjp(ctx.handle, xin.handle, _ptr(ϕ.W), _ptr(ϕ.b), D, ϕ.ACTS[ϕ.act], ϕ.scale,
+                                         C.c_void_p(dphi_ptr), ld_dphi, _ptr(out.get("W")), _ptr(out.get("b")),
+                                         None if dx_ptr is None else C.c_void_p(dx_ptr), max(din, 1)))
+    if "xin" in wrt:
+        if x_torch is not None:
+            import torch
+
+            ctx.release_to_torch_stream(x_torch.device)
+            out["xin"] = dx if dx is not None else torch.empty((0, din), dtype=torch.float64, device=x_torch.device)
+        else:
+            out["xin"] = dx.download().reshape((din, N), order="F") if dx is not None else np.empty((din, 0))
+    return out
 
 
 class TorchFeatureMap:
@@ -375,12 +454,13 @@ GRAD_KEYS = ("X", "y", "σ²", "mw", "Λw")
 
 
 def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatrix, yv, Σy, wrt, out_like=None, k=None,
-                      weights=None):
+                      weights=None, keep_dX=False):
     """One blr_logpdf_grad call, or with `k` one blr_logpdf_multi_grad call: then yv is the device address of Y (N x k,
     column-major, ld = N), the value is the k log densities and the gradients are those of Σ_j weights_j ℓ_j (weights: None for
     all ones).  Per-observation gradients are written into CUDA tensors on out_like's device when `out_like` (a CUDA tensor) is
     given -- dX with the shape torch sees x in, (N, D) for ColVecs; "y" (N, k) -- else downloaded into numpy arrays (dX with the
-    Julia-side shape).  Keys of `wrt` not in GRAD_KEYS are an error; keys left out get NULL."""
+    Julia-side shape; with keep_dX the device buffer itself, ColVecs only).  Keys of `wrt` not in GRAD_KEYS are an error; keys
+    left out get NULL."""
     wrt = tuple(wrt)
     bad = [k for k in wrt if k not in GRAD_KEYS]
     if bad:
@@ -448,6 +528,9 @@ def _logpdf_grad_call(ctx: Context, blr: BayesianLinearRegressor, X: DeviceMatri
         out.update(dev)
     else:
         for key, v in dev.items():
+            if key == "X" and keep_dX:
+                out[key] = v
+                continue
             a = v.download()
             if key == "X":
                 a = a.reshape((D, N) if colv else (N, D), order="F")
@@ -465,7 +548,12 @@ def logpdf_and_grad(fx: FiniteGP, y, wrt=GRAD_KEYS, weights=None):
     ColVecs); otherwise everything is numpy (dX D x N for ColVecs, N x D for RowVecs).
     A matrix `Y` (N x k, a host array or a CUDA tensor; one observation vector per column) returns the k log densities and the
     gradients of Σ_j weights_j ℓ_j (weights: k values, None for all ones) from ONE call (blr_logpdf_multi_grad): the Gram pass and
-    the O(N D²) product run once for all k columns.  "y" then has Y's shape."""
+    the O(N D²) product run once for all k columns.  "y" then has Y's shape.
+    For a BasisFunctionRegressor over AffineFeatures or RandomFourierFeatures, `wrt` may also hold "W" and "b" (the gradients
+    with respect to ϕ's parameters, D x d_in and D numpy) and "xin" (with respect to ϕ's input, shaped as vjp returns it):
+    ∂ℓ/∂ϕ(x) stays on the device and goes through one blr_x_features_vjp call."""
+    if any(k in FEATURE_GRAD_KEYS for k in wrt):
+        return _logpdf_and_feature_grad(fx, y, tuple(wrt), weights)
     fx = _to_finite_blr(fx)
     ctx = fx._context()
     out_like = None
@@ -480,7 +568,36 @@ def logpdf_and_grad(fx: FiniteGP, y, wrt=GRAD_KEYS, weights=None):
     return _logpdf_grad_call(ctx, fx.f, X, yv, fx.Σy, wrt, out_like)
 
 
-def _logpdf_multi_grad(ctx: Context, fx: FiniteGP, Y, wrt, weights, out_like):
+def _logpdf_and_feature_grad(fx: FiniteGP, y, wrt, weights):
+    """logpdf_and_grad through a device feature map: x uploaded and ϕ(x) evaluated once, ∂ℓ/∂ϕ(x) written by blr_logpdf_grad
+    (blr_logpdf_multi_grad for a matrix Y) into a device buffer, then one VJP call."""
+    ϕ = fx.f.ϕ if isinstance(fx.f, BasisFunctionRegressor) else None
+    if not isinstance(ϕ, _DeviceAffineMap):
+        raise L.BLRError(L.E_INVALID, "gradients with respect to \"W\", \"b\" and \"xin\" need a BasisFunctionRegressor over "
+                                      "AffineFeatures or RandomFourierFeatures; differentiate a TorchFeatureMap with torch autograd "
+                                      "(torch_logpdf)")
+    ctx = ϕ._context()
+    xin = ϕ._device_inputs(ctx, fx.x)
+    Φ = ϕ(ColVecs(xin))
+    inner = tuple(k for k in wrt if k not in FEATURE_GRAD_KEYS) + (() if "X" in wrt else ("X",))
+    ffx = FiniteGP(fx.f.blr, Φ, fx.Σy, ctx)
+    out_like = y if _is_torch_cuda(y) else None
+    if (isinstance(y, np.ndarray) or _is_torch_cuda(y)) and y.ndim == 2:
+        lp, g = _logpdf_multi_grad(ctx, ffx, y, inner, weights, out_like, keep_dX=True)
+    else:
+        lp, g = _logpdf_grad_call(ctx, ffx.f, Φ.X, _as_device_vector(ctx, y), fx.Σy, inner, out_like, keep_dX=True)
+    dΦ = g.pop("X")
+    D, N = Φ.X.D, Φ.X.N
+    ptr = dΦ.data_ptr() if out_like is not None else dΦ.device_ptr()
+    if out_like is not None:
+        ctx.wait_torch_stream(dΦ)
+    g.update(_features_vjp(ctx, ϕ, xin, ptr, max(D, 1), [k for k in wrt if k in FEATURE_GRAD_KEYS], _torch_of(fx.x)))
+    if "X" in wrt:
+        g["X"] = dΦ if out_like is not None else dΦ.download().reshape((D, N), order="F")
+    return lp, g
+
+
+def _logpdf_multi_grad(ctx: Context, fx: FiniteGP, Y, wrt, weights, out_like, keep_dX=False):
     X = x_as_colvecs(ctx, fx.x)
     k = int(Y.shape[1])
     if X.D != fx.f.mw.shape[0]:
@@ -494,9 +611,9 @@ def _logpdf_multi_grad(ctx: Context, fx: FiniteGP, Y, wrt, weights, out_like):
 
         Yt = Y.to(torch.float64).T.contiguous()  # (k, N) row-major == N x k column-major
         ctx.wait_torch_stream()
-        return _logpdf_grad_call(ctx, fx.f, X, C.c_void_p(Yt.data_ptr()), fx.Σy, wrt, out_like, k, weights)
+        return _logpdf_grad_call(ctx, fx.f, X, C.c_void_p(Yt.data_ptr()), fx.Σy, wrt, out_like, k, weights, keep_dX)
     Yd = DeviceVector.upload(ctx, np.asarray(Y, dtype=np.float64).T.reshape(-1))  # column-major N x k, flattened
-    return _logpdf_grad_call(ctx, fx.f, X, C.c_void_p(Yd.device_ptr()), fx.Σy, wrt, out_like, k, weights)
+    return _logpdf_grad_call(ctx, fx.f, X, C.c_void_p(Yd.device_ptr()), fx.Σy, wrt, out_like, k, weights, keep_dX)
 
 
 def _torch_logpdf_function():
@@ -597,6 +714,61 @@ def torch_logpdf(X, y, mw, Λw, σ2):
     if _TORCH_LOGPDF is None:
         _TORCH_LOGPDF = _torch_logpdf_function()
     return _TORCH_LOGPDF[1 if y.dim() == 2 else 0].apply(X, y, mw, Λw, σ2)
+
+
+def _torch_features_function():
+    import torch
+
+    class TorchFeatures(torch.autograd.Function):
+        """ϕ(x) = scale * act(W x + b) as a differentiable torch op: forward is blr_x_features, returned as a zero-copy (N, D)
+        view of the library's matrix; only x, W and b are saved; backward is one blr_x_features_vjp call."""
+
+        @staticmethod
+        def forward(fctx, x, W, b, act, scale):
+            if not (x.is_cuda and x.dtype == torch.float64 and x.dim() == 2):
+                raise L.BLRError(L.E_INVALID, "torch_features: x must be an (N, d_in) float64 CUDA tensor")
+            ϕ = _torch_affine_map(W, b, act, scale)
+            fctx.save_for_backward(x, W, b)
+            fctx.act, fctx.scale = act, scale
+            return ϕ(ColVecs(x.detach().contiguous())).X.as_torch()
+
+        @staticmethod
+        def backward(fctx, gΦ):
+            x, W, b = fctx.saved_tensors
+            need = fctx.needs_input_grad
+            wrt = [k for k, n in zip(("xin", "W", "b"), need[:3]) if n]
+            if not wrt:
+                return (None,) * 5
+            ϕ = _torch_affine_map(W, b, fctx.act, fctx.scale)
+            g = ϕ.vjp(ColVecs(x.detach().contiguous()), gΦ.to(torch.float64).contiguous(), wrt)
+            dx = g.get("xin")
+            dW = None if "W" not in g else torch.as_tensor(g["W"], dtype=W.dtype, device=W.device)
+            db = None if "b" not in g else torch.as_tensor(g["b"], dtype=b.dtype, device=b.device)
+            return dx, dW, db, None, None
+
+    return TorchFeatures
+
+
+def _torch_affine_map(W, b, act, scale) -> AffineFeatures:
+    import torch
+
+    return AffineFeatures(W.detach().to("cpu", torch.float64).numpy(), b.detach().to("cpu", torch.float64).numpy(), act, float(scale))
+
+
+_TORCH_FEATURES = None
+
+
+def torch_features(x, W, b, act: str = "cos", scale: float = 1.0):
+    """ϕ(x) = scale * act(W x + b) for an (N, d_in) float64 CUDA tensor x, W (D, d_in) and b (D,), as an (N, D) CUDA tensor that
+    torch autograd differentiates with respect to x, W and b on the device (blr_x_features / blr_x_features_vjp).  Composes with
+    torch_logpdf: torch_logpdf(torch_features(x, Ω / ℓ, b, "cos", (2 / D) ** 0.5), y, mw, Λw, σ²).backward() gives ∂/∂ℓ of
+    a random-Fourier-feature regressor.
+    Against torch autograd of the same map in fp64 this saves memory, not time: it keeps no N x D temporaries (torch's
+    holds several), but its backward is currently about 2x slower (DESIGN.md, K10)."""
+    global _TORCH_FEATURES
+    if _TORCH_FEATURES is None:
+        _TORCH_FEATURES = _torch_features_function()
+    return _TORCH_FEATURES.apply(x, W, b, act, scale)
 
 
 def posterior(fx: FiniteGP, y):

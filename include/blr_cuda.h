@@ -158,6 +158,20 @@ int blr_x_rff(blr_ctx* ctx, const blr_x* xin, const double* W, const double* b, 
 #define BLR_ACT_SIN 4
 int blr_x_features(blr_ctx* ctx, const blr_x* xin, const double* W, const double* b, int64_t D, int act, double scale,
                    blr_x** out);
+/* Vector-Jacobian product of blr_x_features for a cotangent dΦ (what blr_logpdf_grads.dX_dev holds), so gradients reach the
+ * feature map's parameters and inputs (the reference differentiates ϕ with Zygote).  With z_n = W x_n + b and
+ * g_dn = dΦ_dn * scale * act'(z_dn)  (act' = -sin, 1 - tanh², 1[z > 0] (0 at z = 0), 1, cos for COS, TANH, RELU, IDENTITY, SIN):
+ *   dW = Σ_n g_n x_n'  (host, D x d_in column-major, W's layout)    db = Σ_n g_n  (host, D)    dx_n = W' g_n  (device, d_in x N)
+ * W, b, act and scale mean what they mean for blr_x_features (blr_x_rff: act = COS, scale = sqrt(2/D)).
+ *   dphi_dev : device, D x N ColVecs, leading dimension ld_dphi >= D;   dxin_dev : device, d_in x N ColVecs, ld_dxin >= d_in.
+ * Any output may be NULL (not computed); a call that requests nothing launches nothing.  N == 0 writes zeros to dW and db.
+ * BLR_E_INVALID for RowVecs xin, d_in outside 1 .. 384, an unknown act, NULL W / b / dphi_dev, D < 1, or a leading dimension
+ * too small.  z is recomputed (the forward saves nothing) and no N x D workspace is used.  With a communicator dW and db are
+ * summed over ranks (one all-reduce of D (d_in + 1) doubles, D when only db is requested) and replicated; dxin covers this
+ * rank's shard.  Fixed-order sums: repeated
+ * calls are bit-identical. */
+int blr_x_features_vjp(blr_ctx* ctx, const blr_x* xin, const double* W, const double* b, int64_t D, int act, double scale,
+                       const double* dphi_dev, int64_t ld_dphi, double* dW_host, double* db_host, double* dxin_dev, int64_t ld_dxin);
 
 /* ------------------------------------------------------------------ inference
  * replaces __compute_inference_quantities / logpdf / posterior,

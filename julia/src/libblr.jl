@@ -165,6 +165,15 @@ function _download(ctx::Context, h::DeviceVec, n::Integer)
 end
 function logpdf_grad(ctx::Context, prior::Prior, x::DeviceX, layout::Cint, y::DeviceVec, noise::Noise; diagonal::Bool)
     D, N = x.D, x.N
+    lp, hX, _, dy, dσ², dmw, dΛ = logpdf_grad_dev(ctx, prior, x, layout, y, noise; diagonal=diagonal)
+    dX = reshape(_download(ctx, hX, D * N), layout == COLVECS ? (D, N) : (N, D))
+    return lp, dX, dy, dσ², dmw, dΛ
+end
+
+# the same with ∂/∂X left on the device: returns (logpdf, hX (the library-owned vector, keeps the buffer alive), pX (its device
+# address, leading dimension D for ColVecs), dy, dσ², dmw, dΛw) -- what a feature-map rule hands to features_vjp
+function logpdf_grad_dev(ctx::Context, prior::Prior, x::DeviceX, layout::Cint, y::DeviceVec, noise::Noise; diagonal::Bool)
+    D, N = x.D, x.N
     dmw = Vector{Float64}(undef, D)
     dΛ = diagonal ? Vector{Float64}(undef, D) : Matrix{Float64}(undef, D, D)
     dσ²_host = Ref{Float64}(NaN)
@@ -180,9 +189,24 @@ function logpdf_grad(ctx::Context, prior::Prior, x::DeviceX, layout::Cint, y::De
             (Ptr{Cvoid}, Ref{Prior}, Ptr{Cvoid}, Ptr{Cvoid}, Ref{Noise}, Ref{Float64}, Ref{LogpdfGrads}),
             ctx.ptr, prior, x.ptr, y.ptr, noise, lp, g))
     end
-    dX = reshape(_download(ctx, hX, D * N), layout == COLVECS ? (D, N) : (N, D))
     dσ² = vector_noise ? _download(ctx, hs, N) : dσ²_host[]
-    return lp[], dX, _download(ctx, hy, N), dσ², dmw, dΛ
+    return lp[], hX, pX, _download(ctx, hy, N), dσ², dmw, dΛ
+end
+
+# vector-Jacobian product of ϕ(x) = scale * act(W x + b) (blr_x_features_vjp) for the cotangent at device address pdphi (D x N,
+# leading dimension ld_dphi): returns (dW (D x d_in), db (D), dx (d_in x N))
+function features_vjp(ctx::Context, xin::DeviceX, W::Matrix{Float64}, b::Vector{Float64}, act::Integer, scale::Float64,
+                      pdphi::Ptr{Float64}, ld_dphi::Integer)
+    D, din, N = size(W, 1), size(W, 2), xin.N
+    dW = Matrix{Float64}(undef, D, din)
+    db = Vector{Float64}(undef, D)
+    hx, px = _alloc_vec(ctx, din * N)
+    check(ctx, ccall((:blr_x_features_vjp, libblr), Cint,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Cint, Float64, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Int64),
+        ctx.ptr, xin.ptr, W, b, D, act, scale, pdphi, ld_dphi, dW, db, N > 0 ? px : C_NULL, max(din, 1)))
+    dx = N > 0 ? reshape(_download(ctx, hx, din * N), din, N) : zeros(din, 0)
+    return dW, db, dx
 end
 
 # gradients of Σ_j Δ_j logpdf(fx, Y[:, j]) (blr_logpdf_multi_grad): one call for all k columns; Δ is the cotangent of the k

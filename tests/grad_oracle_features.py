@@ -3,7 +3,7 @@ in numpy.  With z = W x + b (D x N) and g = dΦ * scale * act'(z):
 
     dW = g x'      db = Σ_n g_n      dx = W' g
 
-act' is -sin, 1 - tanh², 1[z > 0] (0 at z = 0, as torch and Flux define it), 1 and cos for "cos", "tanh", "relu", "identity" and
+act' is -sin, sech² (evaluated as 4e / (1 + e)², e = exp(-2|z|)), 1[z > 0] (0 at z = 0, as torch and Flux define it), 1 and cos for "cos", "tanh", "relu", "identity" and
 "sin".  tests/test_oracle_grad_features.py pins this against torch autograd and, composed with tests/grad_oracle.py, against
 central differences of the log marginal likelihood.
 """
@@ -25,7 +25,8 @@ def act_grad(z, act):
     if act == "sin":
         return np.cos(z)
     if act == "tanh":
-        return 1.0 - np.tanh(z) ** 2
+        e = np.exp(-2.0 * np.abs(z))  # sech² z = 4e / (1 + e)²: 1 - tanh² z loses every digit by |z| ≈ 19
+        return 4.0 * e / (1.0 + e) ** 2
     if act == "relu":
         return (z > 0.0).astype(np.float64)
     return np.ones_like(z)
